@@ -2,6 +2,7 @@
 """bench.py -- agent-steps/sec of the per-timestep agent update (query + Zanlungo + integrate).
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c3|c4|c2] [--variant ...]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the whole hot path (LocationHash2D rebuild,
 radius query, Zanlungo force, Euler integration) over the synthetic crowd.
@@ -15,6 +16,11 @@ The shuffled crowd is timed in frozen-snapshot mode (RCS_STEP_NO_COMMIT): the re
 a dense mixed bidirectional crowd non-finite within 3-23 steps (SURVEY.md section 0.4), so every timed step
 runs the full pipeline on the same physical snapshot and discards the result.  `--variant lane` times the
 lane-ordered crowd with committed steps instead (force pass idle).
+
+--dump-outputs DIR (one GPU): after the timed steps, the agent state the last timed step produced -- ids, x, y, vx, vy
+in ascending id order, what rcs_read_agents returns to a caller -- goes to DIR/<name>.npy as float64, a fixed
+seeded sample of DUMP_MAX_AGENTS agents for larger crowds.  The inputs are the same in every run with the same
+arguments, so two builds can be compared array for array.
 
 The reference arm (--impl reference) and the cpu_baseline leg time the CPU oracle in its literal
 data-structure form (hash maps, in-loop index update, map iteration order), single-threaded like the
@@ -34,10 +40,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 ALGO_BYTES_ZANLUNGO = 88  # SURVEY.md 8(d): read x,y,vx,vy,pvx,pvy + id, write x,y,vx,vy
 ALGO_BYTES_NOLOCALPLAN = 64
 L2_FLUSH_BYTES = 512 << 20
+DUMP_MAX_AGENTS = 1 << 20  # --dump-outputs: five float64 arrays of at most 2^20 agents, 40 MiB
+DUMP_SEED = 0
 
 
 def measured_peaks():
@@ -245,7 +254,8 @@ def run_gpu_single(args):
     flush = state_bytes < (1 << 30)
 
     clocks = ClockSampler(0)
-    m = timed_steps(sim, n, dt, frozen, args.steps, max(args.warmup, 3), flush, heat_s=0.4, clocks=clocks)
+    m = timed_steps(sim, n, dt, frozen, args.steps, max(args.warmup, 3), flush, heat_s=0.4, clocks=clocks,
+                    keep_state=bool(args.dump_outputs) and not frozen)
     total_ms, K, kt_ms, kt_n, launches, st = m["total_ms"], args.steps, m["kt_ms"], m["kt_n"], m["launches"], m["stats"]
     wall0, wall1 = m["wall0"], m["wall1"]
     value = n * K / (total_ms * 1e-3)
@@ -285,6 +295,14 @@ def run_gpu_single(args):
             roofline["step_dram_bytes"] = counts.get("step_dram_bytes")
             roofline["step_algorithmic_bytes"] = algo * n
 
+    if args.dump_outputs:
+        state = m["state"]
+        if frozen:
+            # the timed steps discarded their result (RCS_STEP_NO_COMMIT) and left the snapshot as it was: one
+            # committed step from that snapshot computes the same step and makes its result readable
+            sim.step(dt)
+            state = sim.read_state()
+        dump_outputs(args.dump_outputs, state)
     sim.spatial_index.close()
     secondary = None if args.skip_secondary else secondary_lines(args, scene, peaks)
     sample_scene, sample = cpu_sample_scene(workload, args.variant, 6)
@@ -315,17 +333,18 @@ def run_gpu_single(args):
     print(json.dumps(line), flush=True)
 
 
-def timed_steps(sim, n, dt, frozen, K, warmup, flush, heat_s=0.0, clocks=None):
+def timed_steps(sim, n, dt, frozen, K, warmup, flush, heat_s=0.0, clocks=None, keep_state=False):
     """W untimed steps (+ optional extra load for the clock samples), then K steps, each bracketed by events on the
-    launching stream with L2 flushed in between when the state is small.  Returns times and counters."""
+    launching stream with L2 flushed in between when the state is small.  Returns times and counters, and with
+    keep_state the agent state right after the K steps."""
     import ctypes as C
 
     from rmf_crowdsim_b200 import _native as N
 
     lib, h = sim._lib, sim._h
 
-    def one_step():
-        N.check(h, lib.rcs_step_async(h, dt.secs, dt.nanos, N.RCS_STEP_NO_COMMIT if frozen else N.RCS_STEP_DEFAULT))
+    def one_step(commit=not frozen):
+        N.check(h, lib.rcs_step_async(h, dt.secs, dt.nanos, N.RCS_STEP_DEFAULT if commit else N.RCS_STEP_NO_COMMIT))
 
     for _ in range(warmup):
         one_step()
@@ -335,9 +354,11 @@ def timed_steps(sim, n, dt, frozen, K, warmup, flush, heat_s=0.0, clocks=None):
     if heat_s > 0:  # keep stepping so that the clock samples are taken under load
         t_end = time.time() + heat_s
         heat = 0
-        while time.time() < t_end and heat < 600:  # 600 committed steps = 13 m of the 64 m margin
+        # The number of these steps depends on the clock: they never commit, so that the timed steps start from the
+        # same state in every run.  An even number of them leaves the handle's buffers as the warm-up left them.
+        while time.time() < t_end and heat < 600:
             for _ in range(8):
-                one_step()
+                one_step(commit=False)
             heat += 8
             sim.sync()
     launches0 = sim.launch_count()
@@ -360,6 +381,7 @@ def timed_steps(sim, n, dt, frozen, K, warmup, flush, heat_s=0.0, clocks=None):
     wall1 = time.perf_counter()
     launches = sim.launch_count() - launches0 - (K if flush else 0)
     stats = sim.stats()
+    state = sim.read_state() if keep_state else None  # before the kernel-timing steps below move the crowd on
     g0 = sim.graph_stats()
     # The dominant kernel, bracketed by its own event pair on the launching stream: a second short pass, because a
     # step with kernel timing on is launched kernel by kernel while the steps above replay as CUDA graphs.
@@ -373,7 +395,19 @@ def timed_steps(sim, n, dt, frozen, K, warmup, flush, heat_s=0.0, clocks=None):
     N.check(h, lib.rcs_kernel_time_ms(h, C.byref(kt_ms), C.byref(kt_n)))
     N.check(h, lib.rcs_kernel_timing(h, 0))
     return {"total_ms": total_ms, "kt_ms": kt_ms.value, "kt_n": kt_n.value, "launches": launches, "stats": stats,
-            "wall0": wall0, "wall1": wall1, "graph_steps": g0[0], "graphs_captured": g0[1]}
+            "wall0": wall0, "wall1": wall1, "graph_steps": g0[0], "graphs_captured": g0[1], "state": state}
+
+
+def dump_outputs(out_dir: str, state: dict) -> None:
+    """ids, x, y, vx, vy (ascending id) as DIR/<name>.npy, float64.  A crowd of more than DUMP_MAX_AGENTS agents is
+    sampled: DUMP_MAX_AGENTS of them drawn with DUMP_SEED, kept in id order, the same agents in every run."""
+    n = len(state["id"])
+    pick = slice(None)
+    if n > DUMP_MAX_AGENTS:
+        pick = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_AGENTS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("id", "x", "y", "vx", "vy"):
+        np.save(os.path.join(out_dir, f"{name}.npy"), state[name][pick].astype(np.float64))
 
 
 def secondary_lines(args, main_scene, peaks) -> list:
@@ -560,11 +594,15 @@ def main():
     ap.add_argument("--skip-verify", action="store_true", help="--gpus N: skip the pre-timing NCCL correctness check")
     ap.add_argument("--verify-dist", action="store_true",
                     help="with --gpus N: committed steps over the NCCL transport compared bit for bit with one handle")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the agent state the last timed step produced to DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "c5" or args.gpus != 1 or world != 1):
+        ap.error("--dump-outputs is implemented for the one-GPU arm only (not --impl reference, --workload c5, --gpus N)")
     if args.impl == "reference":
         run_reference(args)
         return
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.workload == "c5" and args.gpus == 1 and world == 1:
         from rmf_crowdsim_b200 import stream_bench
 

@@ -61,6 +61,13 @@ def test_reference_arm_under_a_launcher_only_rank_0_reports():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_dump_outputs_is_refused_where_it_is_not_implemented(tmp_path):
+    for extra in (("--impl", "reference"), ("--workload", "c5"), ("--gpus", "2")):
+        r = _run(*extra, "--steps", "1", "--warmup", "1", "--dump-outputs", str(tmp_path / "out"))
+        assert r.returncode == 2 and "--dump-outputs" in r.stderr, extra
+    assert not (tmp_path / "out").exists()
+
+
 def test_product_arm_fails_loudly_without_a_cuda_device():
     if _has_cuda_device():
         pytest.skip("a CUDA device is present")
