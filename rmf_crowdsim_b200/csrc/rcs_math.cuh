@@ -110,15 +110,24 @@ __device__ __forceinline__ bool column_cell_range(const GridDev& g, int64_t x, i
 
 // Zanlungo::time_to_collision (zanlungo.rs:49-74) with rel_vel = (rvx, rvy), rel_pos = (rpx, rpy),
 // rp2 = rel_pos.norm_squared() (already computed by the radius filter from the same dx, dy).
-// Early exits are exact (derivations in DESIGN.md "ttc early exits"): a == 0 or NaN => INF;
-// numerator of the larger root <= 0 => both roots <= 0 => INF.  Everything else is literal.
+// Early exits are exact (DESIGN.md section 4.4); everything else is literal, including the division by 2a == +0.
+//  * a == 0 and fl(b*b) == 0 => INF (a NaN a or b*b goes on: the discriminant or both roots are NaN, INF).
+//    With a == 0 and fl(b*b) == 0,
+//    disc = 0 - (0*c) is +-0 (or NaN for a non-finite c), so both numerators are -b and both roots are
+//    -b/+0 of one sign (or NaN): -inf fails every test, +inf is returned as the last root, i.e. INF.
+//    a == 0 ALONE is not an exit: a relative speed below ~1.5e-162 underflows a to 0 while fl(b*b) can be a
+//    non-zero subnormal whose square root exceeds |b|; the reference then divides by +0, gets t0 = -inf,
+//    t1 = +inf and returns 0.
+//  * numerator of the larger root <= 0 => INF.  For a > 0 both roots are <= 0 (n0 <= n1).  For a == 0,
+//    t1 = n1 / +0 is -inf or NaN and t0 = n0 / +0 with n0 <= n1 <= 0 as well: no root is > 0.
 __device__ __forceinline__ double time_to_collision(double rvx, double rvy, double rpx, double rpy, double rp2,
                                                     double rr) {
   double a = rvx * rvx + rvy * rvy;
-  if (!(a > 0.0)) return RCS_INF;
   double b = 2.0 * (rvx * rpx + rvy * rpy);
+  double bb = b * b;
+  if ((__double_as_longlong(a) | __double_as_longlong(bb)) == 0ll) return RCS_INF;  // both +0 (squares: never -0)
   double c = rp2 - rr;
-  double discriminant = b * b - (4.0 * a) * c;
+  double discriminant = bb - (4.0 * a) * c;
   if (discriminant < 0.0) return RCS_INF;
   double sq = sqrt(discriminant);
   double n1 = -b + sq;

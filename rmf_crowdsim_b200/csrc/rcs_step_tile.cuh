@@ -386,11 +386,15 @@ __global__ void __launch_bounds__(32 * ST_WARPS, RCS_TILE_BLOCKS) step_tile_kern
       const double qc = d2 - rr;
       const double bb = qb * qb;
       const double disc = bb - (4.0 * qa) * qc;
-      // A finite time needs a > 0, disc >= 0 and -b + sqrt(disc) > 0.  For b >= 0, disc <= b*b gives
-      // sqrt(disc) <= sqrt(fl(b*b)) = b (correctly rounded sqrt of a square is exact and monotone), so the
-      // numerator is <= 0: INF.  disc == b*b is passed on although it cannot be finite either, so that one
-      // compare also covers b*b = inf.  Everything else is decided by the literal routine on the list.
-      return v && (qa > 0.0) && (disc >= 0.0) && ((qb < 0.0) || !(disc < bb));
+      // A finite time needs a or fl(b*b) != 0 (time_to_collision's first exit: a == 0 alone can still give
+      // t_i = 0), disc >= 0 and -b + sqrt(disc) > 0.  For b >= 0, disc < fl(b*b) means disc <= fl(b*b) - 1 unit,
+      // which is below the exact b^2 (fl(b*b) is within half a unit of it, normal or subnormal), so
+      // sqrt(disc) <= b (correctly rounded sqrt is monotone, b is a double) and the numerator is <= 0: INF.
+      // disc == b*b is passed on: sqrt(fl(b*b)) can exceed b when b*b is subnormal, and the same compare covers
+      // b*b = inf.  Everything else is decided by the literal routine on the list.  a and b*b are +0, positive or
+      // NaN (a NaN fails disc >= 0), so the first test is an integer OR of their bits: no FP64 instruction.
+      return v && ((__double_as_longlong(qa) | __double_as_longlong(bb)) != 0ll) && (disc >= 0.0) &&
+             ((qb < 0.0) || !(disc < bb));
     };
     // Pairs that may return a finite time are queued per warp; slots come from ballots (no atomics, and the count is a
     // register the whole warp agrees on, so nothing is read back from shared memory inside the loop).

@@ -10,6 +10,24 @@ import numpy as np
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 INF = float("inf")
+NAN = float("nan")
+
+
+def _div(x, y):
+    """IEEE-754 x / y, as Rust divides; Python raises on a zero divisor: x / +-0 is +-inf by the signs, 0 / 0 NaN."""
+    if y != 0.0:
+        return x / y
+    if x != x or x == 0.0:
+        return NAN
+    return math.copysign(INF, x) * math.copysign(1.0, y)
+
+
+def _exp(x):
+    """f64::exp: overflows to inf where Python raises."""
+    try:
+        return math.exp(x)
+    except OverflowError:
+        return INF
 
 
 def _norm(v):
@@ -39,11 +57,9 @@ class Zanlungo:
         discriminant = b * b - 4.0 * a * c
         if discriminant < 0.0:
             return INF
-        if a == 0.0:  # 0/0 = NaN in Rust: every comparison below is false
-            return INF
         sq = math.sqrt(discriminant)
-        t0 = (-b - sq) / (2.0 * a)
-        t1 = (-b + sq) / (2.0 * a)
+        t0 = _div(-b - sq, 2.0 * a)  # a == 0 divides by +0: +-inf, or NaN for a zero numerator
+        t1 = _div(-b + sq, 2.0 * a)
         if (t0 < 0.0 and t1 > 0.0) or (t1 < 0.0 and t0 > 0.0):
             return 0.0
         if t0 < t1 and t0 > 0.0:
@@ -101,10 +117,10 @@ class Zanlungo:
         dn = (d_ij[0] / n, d_ij[1] / n) if n != 0.0 else (float("nan"), float("nan"))
         surface_dist = dist - self.agent_radius * 2.0
         rv = (my_vel[0] - other_vel[0], my_vel[1] - other_vel[1])
-        magnitude = weight * self.agent_scale * _norm(rv) / t_i
+        magnitude = _div(weight * self.agent_scale * _norm(rv), t_i)
         if magnitude >= 1e15:
             magnitude = 1e15
-        s = magnitude * math.exp(-surface_dist / self.force_distance)
+        s = magnitude * _exp(_div(-surface_dist, self.force_distance))
         return (dn[0] * s, dn[1] * s)
 
 
@@ -158,6 +174,126 @@ def test_crowd_step_agrees_with_the_independent_restatement():
         vx, vy = pref[0] + fx * (1.0 / 1.0), pref[1] + fy * (1.0 / 1.0)
         assert _rel(vx, g["vx"][i], 1.0) <= 1e-14 and _rel(vy, g["vy"][i], 1.0) <= 1e-14
     assert finite > 100 and worst <= 1e-13
+
+
+def _nx(x, k):
+    """k steps of nextafter from x (toward +inf for k > 0)."""
+    for _ in range(abs(k)):
+        x = math.nextafter(x, INF if k > 0 else -INF)
+    return x
+
+
+# (agent_radius, rel_vel, rel_pos, what) at the edges of time_to_collision (zanlungo.rs:49-74): where a and b*b
+# underflow, where the discriminant is 0 or one unit from it, where the pair touches or overlaps, where b*b
+# overflows, and non-finite components.
+TTC_EDGES = [
+    (0.2, (1.4e-162, 0.0), (1.0, 0.0), "a underflows to 0, b*b subnormal, b > 0: t0 = -inf, t1 = +inf -> 0"),
+    (0.2, (-1.4e-162, 0.0), (1.0, 0.0), "a underflows to 0, b*b subnormal, b < 0 -> 0"),
+    (0.2, (7e-163, 7e-163), (0.8, 0.9), "a == 0, sqrt(fl(b*b)) < b, b > 0: numerator < 0 -> inf"),
+    (0.2, (-7e-163, -7e-163), (0.8, 0.9), "a == 0, sqrt(fl(b*b)) < |b|, b < 0: both roots +inf -> inf"),
+    (0.2, (1e-163, 0.0), (-1.0, 0.0), "a == 0, b*b == 0, b != 0"),
+    (0.2, (0.0, 0.0), (1.0, 0.0), "a == 0, b == 0"),
+    (0.2, (0.0, -0.0), (0.1, 0.0), "a == 0, b == 0, overlapping"),
+    (0.2, (1e-160, 0.0), (-1.0, 0.0), "a subnormal > 0, approaching"),
+    (0.2, (1e-160, 0.0), (1.0, 0.0), "a subnormal > 0, receding"),
+    (0.2, (3e-155, 0.0), (-1.0, 0.0), "a and b*b tiny but normal"),
+    (0.5, (-1.0, 0.0), (3.0, 0.5), "grazing: disc == 0 exactly, t = 3"),
+    (0.5, (-1.0, 0.0), (3.0, _nx(0.5, -17)), "disc one unit of b*b = 36 above 0"),
+    (0.5, (-1.0, 0.0), (3.0, _nx(0.5, 9)), "disc one unit of b*b = 36 below 0"),
+    (0.5, (-1.0, 0.0), (0.5, 0.0), "touching: c == 0"),
+    (0.5, (1.0, 0.0), (0.5, 0.0), "touching, receding"),
+    (0.5, (-1.0, 0.0), (0.3, 0.0), "overlap: c < 0 -> 0"),
+    (0.5, (0.0, 1e-150), (0.3, 0.0), "overlap, tiny perpendicular speed -> 0"),
+    (1e100, (1e60, 0.0), (-1e100, 0.0), "b*b overflows to inf, c == 0: disc = inf"),
+    (0.2, (1e150, 0.0), (-1e10, 0.0), "b*b and 4ac overflow: disc NaN"),
+    (0.2, (1e200, 0.0), (-1.0, 0.0), "a overflows to inf"),
+    (0.2, (INF, 0.0), (-1.0, 0.0), "relative velocity inf"),
+    (0.2, (NAN, 0.0), (-1.0, 0.0), "relative velocity NaN"),
+    (0.2, (-1.0, 0.0), (INF, 0.0), "relative position inf"),
+    (0.2, (-1.0, 0.0), (NAN, 1.0), "relative position NaN"),
+    (0.0, (-1.0, 0.0), (1.0, 0.0), "radius 0"),
+]
+
+
+def _bits(x):
+    return int(np.float64(x).view(np.uint64))
+
+
+def _same_force(f, g):
+    """Components: identical NaN / inf patterns and signs, finite values within the pair-table tolerance."""
+    mag = math.hypot(g[0], g[1]) if all(math.isfinite(v) for v in g) else 0.0
+    for a, b in zip(f, g):
+        if math.isnan(a) or math.isnan(b) or math.isinf(a) or math.isinf(b):
+            if not ((math.isnan(a) and math.isnan(b)) or a == b):
+                return False
+        elif _rel(a, b, mag) > 1e-14:
+            return False
+    return True
+
+
+def test_time_to_collision_edges_agree_with_the_independent_restatement():
+    """Every edge class of time_to_collision bit for bit, and the force of each such pair (both id orders: the yield
+    and the weight-0 branch of right_of_way_vel) at the existing tolerance, NaN and inf patterns included."""
+    import oracle_ffi as O
+
+    L = O.lib()
+    results = set()
+    for r, rv, rp, what in TTC_EDGES:
+        want = O.ttc(r, rv, rp)
+        got = Zanlungo(1, 1, 0, 1, 1, r).time_to_collision(rv, rp)
+        assert _bits(got) == _bits(want), (what, got, want)
+        results.add(want if want == want else "nan")
+        params = np.array([0.05, 1.0, 0.0, 0.5, 1.0, r])
+        z = Zanlungo(*params.tolist())
+        me = (0.25, -0.5, 0.3, 0.1, 1.3, 0.0)  # x, y, vx, vy, preferred vx, vy
+        other = (me[0] + rp[0], me[1] + rp[1], me[2] + rv[0], me[3] + rv[1], 0.0, 0.0)
+        for aid, oid in ((3, 7), (7, 3)):
+            out = np.zeros(2)
+            a, o = np.array(me), np.array(other)
+            L.orc_agent_force(params.ctypes.data_as(O.f64p), aid, a.ctypes.data_as(O.f64p), oid,
+                              o.ctypes.data_as(O.f64p), want, out.ctypes.data_as(O.f64p))
+            f = z.compute_agent_force((aid, me[:2], me[2:4], me[4:]), (oid, other[:2], other[2:4], other[4:]), want)
+            assert _same_force(f, tuple(out)), (what, aid, f, tuple(out))
+    # the table reaches every kind of result: 0, finite > 0, inf
+    assert 0.0 in results and INF in results and any(isinstance(t, float) and 0.0 < t < INF for t in results)
+    # the classes are what their names say
+    assert O.ttc(0.2, (1.4e-162, 0.0), (1.0, 0.0)) == 0.0 and O.ttc(0.5, (-1.0, 0.0), (3.0, 0.5)) == 3.0
+    unit = math.ulp(36.0)
+    for y, disc in ((0.5, 0.0), (_nx(0.5, -17), unit), (_nx(0.5, 9), -unit)):
+        assert 36.0 - 4.0 * ((9.0 + y * y) - 0.25) == disc, y
+
+
+def test_underflowing_relative_speed_gives_t_i_zero_and_a_nan_force():
+    """Two agents 1 m apart whose parity velocities (+-7e-163 m/s) make |v_rel|^2 underflow to 0 while (2 v.p)^2 is a
+    non-zero subnormal: the reference divides by 2a = +0 and returns t_i = 0 (zanlungo.rs:60-70), and the force
+    (2 scale |v|) / 0 is NaN.  Positions go NaN in the second step and stay NaN."""
+    import oracle_ffi as O
+
+    za = (0.05, 1.0, 0.0, 0.5, 1.0, 0.2)
+    o = O.OracleSim(16.0, 16.0, 2.0, (0.0, 0.0))
+    o.add_agents(np.array([[5.0, 5.0], [6.0, 5.0]]), o.hl_parity((7e-163, 0.0)), o.lp_zanlungo(*za), 2.0)
+    o.enable_trace(True)
+    z = Zanlungo(*za)
+    want_t = [[INF, INF], [0.0, 0.0], None]
+    for step in range(3):
+        s = o.read_state()
+        o.step(0, 16_666_667)
+        t = o.read_trace()
+        xy, v = np.stack([s["x"], s["y"]], axis=1), np.stack([s["vx"], s["vy"]], axis=1)
+        for i, j in ((0, 1), (1, 0)):
+            ti = z.time_to_collision((v[j, 0] - v[i, 0], v[j, 1] - v[i, 1]), (xy[j, 0] - xy[i, 0], xy[j, 1] - xy[i, 1]))
+            if math.isnan(xy[i, 0]):
+                continue  # the NaN agents sit in cell 0 and no longer see each other
+            assert _bits(ti) == _bits(t["t_i"][i]), (step, i)
+            if ti != INF:
+                pref = (-7e-163, 0.0) if i % 2 == 0 else (7e-163, 0.0)
+                f = z.compute_agent_force((i, tuple(xy[i]), tuple(v[i]), pref), (j, tuple(xy[j]), tuple(v[j]), (0, 0)),
+                                          ti)
+                assert math.isnan(f[0]) and math.isnan(t["fx"][i]), (step, i)
+        if want_t[step] is not None:
+            assert [_bits(x) for x in t["t_i"]] == [_bits(x) for x in want_t[step]], step
+    s = o.read_state()
+    assert np.isnan(s["x"]).all() and np.isnan(s["y"]).all()
 
 
 class _Hash2D:
