@@ -121,6 +121,7 @@ extern "C" {
     pub fn rcs_nccl_unique_id(out_id: *mut u8) -> c_int;
     pub fn rcs_dist_init(sim: *mut rcs_sim, rank: i32, world: i32, nccl_id: *const u8, halo_capacity: u64) -> c_int;
     pub fn rcs_dist_set_boundaries(sim: *mut rcs_sim, world: i32, bounds: *const u64) -> c_int;
+    pub fn rcs_dist_reserve_ids(sim: *mut rcs_sim, next_id: u64) -> c_int;
     pub fn rcs_dist_peer_export(sim: *mut rcs_sim, out_handle: *mut u8) -> c_int;
     pub fn rcs_dist_peer_connect(sim: *mut rcs_sim, left_handle: *const u8, right_handle: *const u8) -> c_int;
     pub fn rcs_dist_peer_disable(sim: *mut rcs_sim) -> c_int;

@@ -309,6 +309,10 @@ int rcs_dist_strip(rcs_sim* sim, int32_t rank, int32_t world, uint64_t* c0, uint
  * tables are dense over the id range). */
 int rcs_dist_add_agents(rcs_sim* sim, uint64_t n, const uint64_t* ids, const double* xy, const double* vxy,
                         uint32_t hl, uint32_t lp, double eyesight);
+/* The ids source sinks allocate on this handle (lib.rs:128-129) start at next_id or later.  After rcs_dist_add_agents,
+ * every rank calls it with the same value -- one past the largest id the host program has handed out -- so that the
+ * ranks number their spawns alike and after the caller's agents.  next_id < 2^32. */
+int rcs_dist_reserve_ids(rcs_sim* sim, uint64_t next_id);
 /* Single-process transport: sims[r] is rank r of `world` handles that live in this process (on one
  * or several devices); halos move with peer copies ordered by events.  The group is stepped as a
  * whole; rcs_sync / rcs_read_agents / rcs_step_stats work per handle.  Used to test strips on one

@@ -138,6 +138,20 @@ int orc_set_preferred_velocity(void* h, int hl, uint64_t n, const uint64_t* ids,
   return 0;
 }
 
+// HighLevelPlanner::set_target(agent, (0, 0), (0, 0)) for agents addressed by id (the route follower ignores the
+// point: rcs_hl_route_set_target).
+int orc_hl_set_target(void* h, int hl, uint64_t n, const uint64_t* ids) {
+  auto* s = static_cast<OrcSim*>(h);
+  auto& p = s->hls.at(hl);
+  for (uint64_t i = 0; i < n; ++i) {
+    auto it = s->sim->agents.find(ids[i]);
+    if (it == s->sim->agents.end()) return 1;
+    std::lock_guard<std::mutex> g(*p.mtx);
+    p.ptr->set_target(it->second, Vec2{0.0, 0.0}, Vec2{0.0, 0.0});
+  }
+  return 0;
+}
+
 int orc_add_source_sink(void* h, double sx, double sy, double radius_sink, double monotonic_rate, int hl, int lp,
                         uint64_t n_wp, const double* wp_xy, int loop_forever, double eyesight, uint64_t* out_id) {
   auto* s = static_cast<OrcSim*>(h);

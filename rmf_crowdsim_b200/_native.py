@@ -142,6 +142,7 @@ SIGNATURES = {
     "rcs_dist_step_local": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_uint64, C.c_uint32, C.c_uint32]),
     "rcs_dist_strip": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_u64p, c_u64p]),
     "rcs_dist_set_boundaries": (C.c_int, [C.c_void_p, C.c_int32, c_u64p]),
+    "rcs_dist_reserve_ids": (C.c_int, [C.c_void_p, C.c_uint64]),
     "rcs_dist_peer_export": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint8)]),
     "rcs_dist_peer_connect": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint8), C.POINTER(C.c_uint8)]),
     "rcs_dist_peer_disable": (C.c_int, [C.c_void_p]),

@@ -95,10 +95,11 @@ struct StepKey {
   uint64_t epoch = 0, dt_bits = 0;
   const void* cur_pos = nullptr;
   uint32_t flags = 0, n_ub = 0, n = 0;
+  uint32_t n_ub_spawn = 0;  // the launch bound after this step's spawns: phase B's grids (spawn_launch_bound)
   bool cur_has_dead = false, binned_ahead = false;
   bool operator==(const StepKey& o) const {
     return epoch == o.epoch && dt_bits == o.dt_bits && cur_pos == o.cur_pos && flags == o.flags && n_ub == o.n_ub &&
-           n == o.n && cur_has_dead == o.cur_has_dead && binned_ahead == o.binned_ahead;
+           n == o.n && n_ub_spawn == o.n_ub_spawn && cur_has_dead == o.cur_has_dead && binned_ahead == o.binned_ahead;
   }
 };
 struct StepGraph {

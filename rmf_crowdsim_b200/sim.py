@@ -308,6 +308,7 @@ class Simulation:
         self._host_hl: Dict[int, HighLevelPlanner] = {}  # agent id -> host-evaluated planner
         self._host_hl_handle: Optional[int] = None
         self._host_ss: Dict[Tuple[float, float], SourceSink] = {}  # source position -> sink with a host planner
+        self._host_ss_of: Dict[int, SourceSink] = {}  # agent id -> the sink that spawned it (host planners only)
         self._eyesight: Dict[int, float] = {}
         self._listeners: Dict[int, EventListener] = {}
         self._listener_counter = 0
@@ -407,6 +408,7 @@ class Simulation:
     def remove_agents(self, agent: AgentId) -> None:
         ids = _u64([agent])
         N.check(self._h, self._lib.rcs_remove_agents(self._h, 1, _p(ids, N.c_u64p)))
+        self._host_ss_of.pop(int(agent), None)
         hl = self._host_hl.pop(int(agent), None)
         if hl is not None:
             hl.remove_agent_id(int(agent))
@@ -416,10 +418,9 @@ class Simulation:
     # -- lib.rs:195-383 ------------------------------------------------------------------------
     def step(self, dur: Duration) -> None:
         """Err(String) of the reference becomes CrowdsimError with the same message."""
-        if self._host_hl:
-            self._run_host_planners()
+        before = self._run_host_planners() if self._host_hl else None
         N.check(self._h, self._lib.rcs_step(self._h, int(dur.secs), int(dur.nanos)))
-        self._dispatch_events()
+        self._dispatch_events(before)
 
     def step_in_loop(self, dur: Duration, order=None, max_sweeps: int = 0) -> int:
         """One step under the reference's in-loop index semantic (lib.rs:299; SURVEY.md 8f-4) for the iteration order
@@ -443,7 +444,8 @@ class Simulation:
     def sync(self) -> None:
         N.check(self._h, self._lib.rcs_sync(self._h))
 
-    def _run_host_planners(self) -> None:
+    def _run_host_planners(self) -> Dict[str, np.ndarray]:
+        """Uploads the host planners' preferred velocities; returns the pre-step state it read."""
         st = self.read_state()
         ids = st["id"]
         sel, vxy = [], []
@@ -460,17 +462,24 @@ class Simulation:
             vxy.append((nan, nan) if v is None else (float(v[0]), float(v[1])))
         if sel:
             self.set_preferred_velocity(np.array(sel, dtype=np.uint64), np.array(vxy, dtype=np.float64))
+        return st
 
-    def _dispatch_events(self) -> None:
+    def _dispatch_events(self, before: Optional[Dict[str, np.ndarray]] = None) -> None:
+        """Spawn events, then set_target for the host-planned agents that reached an intermediate waypoint in the step
+        (`before`: the state the step started from), then destroy events -- the reference's order (lib.rs:242-249,
+        :326-333, :378-380)."""
         ns, nd = C.c_uint64(), C.c_uint64()
         N.check(self._h, self._lib.rcs_poll_events(self._h, 0, None, None, C.byref(ns), 0, None, C.byref(nd)))
         if ns.value == 0 and nd.value == 0:
+            if before is not None and self._host_ss_of:
+                self._host_waypoint_targets(before, {})
             return
         sid = np.zeros(max(ns.value, 1), dtype=np.uint64)
         sxy = np.zeros(2 * max(ns.value, 1), dtype=np.float64)
         did = np.zeros(max(nd.value, 1), dtype=np.uint64)
         N.check(self._h, self._lib.rcs_poll_events(self._h, len(sid), _p(sid, N.c_u64p), _p(sxy, N.c_f64p),
                                                    C.byref(ns), len(did), _p(did, N.c_u64p), C.byref(nd)))
+        spawned: Dict[int, Point] = {}  # host-planned agents spawned in this step
         for k in range(ns.value):
             pos = (float(sxy[2 * k]), float(sxy[2 * k + 1]))
             ss = self._host_ss.get(pos) if self._host_ss else None
@@ -481,17 +490,47 @@ class Simulation:
                 # host-evaluated planners only, INTEGRATION.md).
                 hl = ss.high_level_planner
                 self._host_hl[int(sid[k])] = hl
+                self._host_ss_of[int(sid[k])] = ss
                 wp0 = ss.waypoints[0]
                 hl.set_target(Agent(int(sid[k]), pos, (0.0, 0.0), 0), (float(wp0[0]), float(wp0[1])),
                               (float(ss.radius_sink), float(ss.radius_sink)))
+                spawned[int(sid[k])] = pos
             for key in sorted(self._listeners):
                 self._listeners[key].agent_spawned(pos, int(sid[k]))
+        if before is not None and self._host_ss_of:
+            self._host_waypoint_targets(before, spawned)
         for k in range(nd.value):
+            self._host_ss_of.pop(int(did[k]), None)
             hl = self._host_hl.pop(int(did[k]), None)
             if hl is not None:
                 hl.remove_agent_id(int(did[k]))
             for key in sorted(self._listeners):
                 self._listeners[key].agent_destroyed(int(did[k]))
+
+    def _host_waypoint_targets(self, before: Dict[str, np.ndarray], spawned: Dict[int, Point]) -> None:
+        """lib.rs:326-333: an agent whose next_waypoint advanced k -> k + 1 in the step gets set_target(agent,
+        waypoints[k + 1], (radius_sink, radius_sink)), with the agent as the step found it, in ascending id.  The loop
+        wrap (last -> 0) calls nothing; agents removed in the step are no longer in the state and get no call."""
+        after = self.read_state()
+        pre = {int(a): k for k, a in enumerate(before["id"])}
+        for k, a in enumerate(after["id"]):
+            a = int(a)
+            ss = self._host_ss_of.get(a)
+            if ss is None:
+                continue
+            j = pre.get(a)
+            if j is not None:
+                agent = Agent(a, (float(before["x"][j]), float(before["y"][j])),
+                              (float(before["vx"][j]), float(before["vy"][j])), int(before["next_waypoint"][j]))
+            elif a in spawned:  # spawned in this step: it starts at the source, at rest, heading for waypoint 0
+                agent = Agent(a, spawned[a], (0.0, 0.0), 0)
+            else:
+                continue
+            wp = int(after["next_waypoint"][k])
+            if wp == agent.next_waypoint + 1:
+                p = ss.waypoints[wp]
+                ss.high_level_planner.set_target(agent, (float(p[0]), float(p[1])),
+                                                 (float(ss.radius_sink), float(ss.radius_sink)))
 
     # -- the pub `agents` field (lib.rs:71) ----------------------------------------------------
     def agent_count(self) -> int:

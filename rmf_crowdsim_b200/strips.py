@@ -132,6 +132,8 @@ class StripSimulation(S.Simulation):
             xy, vxy, ids = scene.xy, scene.vxy, np.arange(scene.n, dtype=np.uint64)
         m = owned_mask(xy[:, 0], scene.offset[0], scene.cell, self.c0, self.c1)
         add_agents_with_ids(self, ids[m], xy[m], None if vxy is None else vxy[m], hl, lp, scene.eyesight)
+        if len(ids):  # source sinks number their spawns after every rank's agents
+            N.check(self._h, self._lib.rcs_dist_reserve_ids(self._h, int(np.max(ids)) + 1))
         return int(m.sum())
 
 
@@ -174,6 +176,7 @@ class LocalStripGroup:
             hl, lp = _planners(scene)
             sm._scene_planners = (hl, lp)
             add_agents_with_ids(sm, ids[m], scene.xy[m], scene.vxy[m], hl, lp, scene.eyesight)
+            N.check(sm._h, self._lib.rcs_dist_reserve_ids(sm._h, scene.n))  # spawned ids follow the scene's agents
             self.counts.append(int(m.sum()))
         assert sum(self.counts) == scene.n
 

@@ -43,6 +43,7 @@ def lib() -> C.CDLL:
             f.argtypes = [C.c_void_p, C.c_double, C.c_double]
         L.orc_hl_host.argtypes = [C.c_void_p]
         L.orc_hl_route.argtypes = [C.c_void_p, C.c_uint64, f64p]
+        L.orc_hl_set_target.argtypes = [C.c_void_p, C.c_int, C.c_uint64, u64p]
         L.orc_add_agents.argtypes = [C.c_void_p, C.c_uint64, f64p, C.c_int, C.c_int, C.c_double, u64p]
         L.orc_remove_agent.argtypes = [C.c_void_p, C.c_uint64]
         L.orc_set_state.argtypes = [C.c_void_p, C.c_uint64, u64p, f64p, f64p, f64p, f64p]
@@ -135,6 +136,12 @@ class OracleSim:
     def hl_route(self, route):
         r = np.ascontiguousarray(route, dtype=np.float64).reshape(-1, 2)
         return self.L.orc_hl_route(self.h, r.shape[0], _p(r, f64p))
+
+    def hl_set_target(self, hl, ids):
+        """set_target on planner `hl` for the given agents (Simulation.route_set_target)."""
+        ids = np.ascontiguousarray(ids, dtype=np.uint64)
+        if self.L.orc_hl_set_target(self.h, hl, len(ids), _p(ids, u64p)):
+            raise OracleError(1, "unknown agent id")
 
     def add_agents(self, xy, hl, lp, eyesight):
         xy = np.ascontiguousarray(xy, dtype=np.float64).reshape(-1, 2)

@@ -4,12 +4,123 @@ cell assignments and neighbour sets bit-exact, t_i bit-exact (only IEEE +,-,*,/,
 forces / velocities <= 1e-9 relative (CUDA's exp/asin/sin differ from glibc's by <= 2 ulp)."""
 from __future__ import annotations
 
+import math
+
 import numpy as np
 
 import oracle_ffi as O
 from rmf_crowdsim_b200 import scenes as SC
 
 REL_TOL = 1e-9
+INF, NAN = float("inf"), float("nan")
+
+
+def _nx(x, k):
+    """k steps of nextafter from x (toward +inf for k > 0)."""
+    for _ in range(abs(k)):
+        x = math.nextafter(x, INF if k > 0 else -INF)
+    return x
+
+
+def radius_threshold(r):
+    """Smallest double T with sqrt(T) >= r (r > 0 finite): sqrt(d2) < r <=> d2 < T."""
+    t = r * r
+    while math.sqrt(t) >= r:
+        t = math.nextafter(t, 0.0)
+    while math.sqrt(t) < r:
+        t = math.nextafter(t, INF)
+    return t
+
+
+def threshold_points(r, x, diagonal, m_max=400):
+    """A probe at (x, -dy/2) and neighbours near (x + dx, +dy/2) -- along the x axis (dy ~ 0.05 r) or the diagonal --
+    at which the computed fl(dx*dx + dy*dy) (dx = fl(qx - px), dy = fl(qy - py)) is T(r) - 1 ulp, T(r) and T(r) + 1 ulp;
+    found by stepping qy (and, where that skips a target, qx) with nextafter.  y stays near 0, where the steps are
+    finer than one unit of T."""
+    t = radius_threshold(r)
+    ang = math.pi / 4 if diagonal else 0.05
+    p = np.array([x, -0.5 * r * math.sin(ang)])
+    targets = (math.nextafter(t, 0.0), t, math.nextafter(t, INF))
+    for k in range(64):
+        qx = _nx(x + r * math.cos(ang), (k + 1) // 2 * (-1) ** k)
+        y0 = np.float64(p[1] + math.sqrt(t - (qx - p[0]) ** 2))  # aim at T with the dx the rounding of qx left
+        ys = (y0.view(np.int64) + np.arange(-m_max, m_max + 1)).view(np.float64)  # consecutive doubles (y0 > 0)
+        dx, dy = qx - p[0], ys - p[1]
+        d2 = dx * dx + dy * dy
+        hits = [np.nonzero(d2 == tg)[0] for tg in targets]
+        if all(len(h) for h in hits):
+            return p, [np.array([qx, ys[h[len(h) // 2]]]) for h in hits]
+    raise AssertionError((r, x, diagonal))
+
+
+PROBE_RADIUS = 0.4  # the spawn probe's hard-coded radius (lib.rs:214)
+CELLS = [(0.3, (0.0, 0.0)), (0.7, (-7.7, 13.1)), (1.1, (0.0, 0.0)), (2.6, (-7.7, 13.1))]
+SINK_RADII = [0.3, 0.6, 1.1, 0.5, 2.0]  # r*r inexact, then exact
+
+
+def probe_threshold_configs(x0=5.0, spacing=11.0):
+    """(source, agent, blocked): an agent at T(0.4) - 1 ulp, T and T + 1 ulp from a source (the computed fl(dx*dx +
+    dy*dy)), along an axis and a diagonal; only T - 1 ulp blocks.  Sources `spacing` apart along y ~ 0."""
+    out, x = [], x0
+    for diagonal in (False, True):
+        for which in range(3):
+            p, qs = threshold_points(PROBE_RADIUS, x, diagonal)
+            out.append((p, qs[which], which == 0))
+            x += spacing
+    return out
+
+
+PROBE_EDGE_ULPS = [(0, 0), (1, 0), (-1, 0), (0, 1), (0, -1), (1, 1), (-1, -1), (2, -2), (-2, 2), (4, -1), (-4, 1),
+                   (8, 8), (-8, -8), (3, -5), (-3, 5), (6, 0)]
+
+
+def probe_edge_configs(cell, off, k0=3, stride=6, row=5):
+    """(source, agent) pairs at the spawn probe's stencil edges: source +- 0.4 within a few ulps of the cell edge
+    e = k*cell + off (so that the stencil's last column ends there) and the agent within a few ulps of e on the same
+    row (column) -- inside or just outside the 0.4 m, in the stencil's edge column or the next.  Right and left edge,
+    along x and along y; pairs `stride` cells apart, isolated from each other."""
+    out, k = [], k0
+    for axis in (0, 1):
+        other = (row + 0.5) * cell + off[1 - axis]
+        for side in (1, -1):  # source + 0.4 (right / top edge) or source - 0.4 (left / bottom edge)
+            for us, ua in PROBE_EDGE_ULPS:
+                e = k * cell + off[axis]
+                s = _nx(e - side * PROBE_RADIUS, us)
+                a = _nx(e, ua)
+                src, ag = [0.0, 0.0], [0.0, 0.0]
+                src[axis], ag[axis] = s, a
+                src[1 - axis] = ag[1 - axis] = other
+                out.append((np.array(src), np.array(ag)))
+                k += stride
+    return out
+
+
+def sink_threshold_configs(x0=5.0, spacing=11.0):
+    """(r, waypoint, agent, inside): agents at T(r) - 1 ulp, T and T + 1 ulp from a waypoint, along an axis and a
+    diagonal, for every radius of SINK_RADII; only T - 1 ulp is `norm < r`."""
+    out, x = [], x0
+    for r in SINK_RADII:
+        for diagonal in (False, True):
+            for which in range(3):
+                p, qs = threshold_points(r, x, diagonal)
+                out.append((r, p, qs[which], which == 0))
+                x += spacing
+    return out
+
+
+def _bits(a):
+    """Bit patterns, every NaN as the one quiet NaN: the sign of a NaN that an arithmetic operation produces is not
+    specified by IEEE 754 (nor used by the reference), and the forms reach the same NaN through different operations."""
+    if a.dtype != np.float64:
+        return a
+    return np.where(np.isnan(a), np.float64(NAN), a).view(np.uint64)
+
+
+def _same(ta, tb, keys):
+    for k in keys:
+        a, b = _bits(ta[k]), _bits(tb[k])
+        bad = np.nonzero(a != b)[0] if a.shape == b.shape else []
+        assert a.shape == b.shape and len(bad) == 0, (k, [(int(i), hex(int(a[i])), hex(int(b[i]))) for i in bad[:8]])
 
 
 def build_oracle(scene: SC.Scene, index_mode=O.DEFERRED, inject_velocity=True) -> O.OracleSim:

@@ -15,6 +15,7 @@ import rmf_crowdsim_b200 as R
 from rmf_crowdsim_b200 import _native as N
 from rmf_crowdsim_b200 import scenes as SC
 from rmf_crowdsim_b200.strips import LocalStripGroup
+from parity import _nx, _same, threshold_points
 
 pytestmark = pytest.mark.gpu
 
@@ -22,22 +23,6 @@ INF, NAN = float("inf"), float("nan")
 ZA = (0.05, 1.0, 0.0, 0.5, 1.0, 0.2)
 HEAVY = (0.05, 1.0, 0.0, 0.5, 50.0, 0.05)  # heavy, small agents: a crowd that stays sane for a few steps
 DT = (0, 16_666_667)
-
-
-def _nx(x, k):
-    for _ in range(abs(k)):
-        x = math.nextafter(x, INF if k > 0 else -INF)
-    return x
-
-
-def radius_threshold(r):
-    """Smallest double T with sqrt(T) >= r (r > 0 finite): sqrt(d2) < r <=> d2 < T."""
-    t = r * r
-    while math.sqrt(t) >= r:
-        t = math.nextafter(t, 0.0)
-    while math.sqrt(t) < r:
-        t = math.nextafter(t, INF)
-    return t
 
 
 class Layout:
@@ -86,21 +71,6 @@ class Layout:
         g.set_option(N.RCS_OPT_STEP_KERNEL, kernel)
         g.set_trace(True)
         return g
-
-
-def _bits(a):
-    """Bit patterns, every NaN as the one quiet NaN: the sign of a NaN that an arithmetic operation produces is not
-    specified by IEEE 754 (nor used by the reference), and the forms reach the same NaN through different operations."""
-    if a.dtype != np.float64:
-        return a
-    return np.where(np.isnan(a), np.float64(NAN), a).view(np.uint64)
-
-
-def _same(ta, tb, keys):
-    for k in keys:
-        a, b = _bits(ta[k]), _bits(tb[k])
-        bad = np.nonzero(a != b)[0] if a.shape == b.shape else []
-        assert a.shape == b.shape and len(bad) == 0, (k, [(int(i), hex(int(a[i])), hex(int(b[i]))) for i in bad[:8]])
 
 
 def _check_forms(lay, steps=1, in_loop=False):
@@ -235,27 +205,6 @@ def test_ttc_edge_classes_match_the_oracle_on_every_kernel_form():
 
 # ---- 2. radius threshold -------------------------------------------------------------------------------------------
 EYESIGHTS = [1.1, 0.3, 1.7, 2.7, 4.1, 0.5, 2.0]  # R*R inexact, then exact
-
-
-def threshold_points(r, x, diagonal, m_max=400):
-    """A probe at (x, -dy/2) and neighbours near (x + dx, +dy/2) -- along the x axis (dy ~ 0.05 r) or the diagonal --
-    at which the computed fl(dx*dx + dy*dy) (dx = fl(qx - px), dy = fl(qy - py)) is T(r) - 1 ulp, T(r) and T(r) + 1 ulp;
-    found by stepping qy (and, where that skips a target, qx) with nextafter.  y stays near 0, where the steps are
-    finer than one unit of T."""
-    t = radius_threshold(r)
-    ang = math.pi / 4 if diagonal else 0.05
-    p = np.array([x, -0.5 * r * math.sin(ang)])
-    targets = (math.nextafter(t, 0.0), t, math.nextafter(t, INF))
-    for k in range(64):
-        qx = _nx(x + r * math.cos(ang), (k + 1) // 2 * (-1) ** k)
-        y0 = np.float64(p[1] + math.sqrt(t - (qx - p[0]) ** 2))  # aim at T with the dx the rounding of qx left
-        ys = (y0.view(np.int64) + np.arange(-m_max, m_max + 1)).view(np.float64)  # consecutive doubles (y0 > 0)
-        dx, dy = qx - p[0], ys - p[1]
-        d2 = dx * dx + dy * dy
-        hits = [np.nonzero(d2 == tg)[0] for tg in targets]
-        if all(len(h) for h in hits):
-            return p, [np.array([qx, ys[h[len(h) // 2]]]) for h in hits]
-    raise AssertionError((r, x, diagonal))
 
 
 def threshold_layout(rng):

@@ -512,3 +512,73 @@ def test_source_sink_stream_agrees_with_the_independent_restatement():
     ids = sorted(agents)
     assert ids == [int(v) for v in g["final_id"]]
     assert [agents[i][0][0] for i in ids] == [float(v) for v in g["final_x"]]
+
+
+def test_spawn_probe_edges_agree_with_the_independent_hash_grid():
+    """The spawn probe `get_neighbours_in_radius(0.4, source)` (lib.rs:212-214) through the second hash-grid
+    restatement and the oracle's index: agents at T(0.4) - 1 ulp, T and T + 1 ulp from a source, and agents next to the
+    probe stencil's edge cell for sources whose +-0.4 lands a few ulps from a cell edge (cells of 0.3, 0.7, 1.1 and
+    2.6 m, with offsets).  Also the claim that no agent within 0.4 m is inserted outside the stencil: floor and the
+    truncating insert agree on non-negative values and rounding is monotone, so `fl(source + 0.4) >= agent` whenever
+    `norm(agent - source) < 0.4`."""
+    import oracle_ffi as O
+    import parity as P
+
+    groups = [(P.probe_threshold_configs(), 2.0, (0.0, -32.0), 80.0, 64.0)]
+    groups += [([(s, a, None) for s, a in P.probe_edge_configs(cell, off)], cell, off, 400 * cell, 400 * cell)
+               for cell, off in P.CELLS]
+    blocked_edge = free_edge = edge_column = 0
+    for configs, cell, off, w, hgt in groups:
+        h = _Hash2D(w, hgt, cell, off)
+        o = O.OracleSim(w, hgt, cell, off)
+        for i, (_, a, _) in enumerate(configs):
+            h.add_or_update(i, (a[0], a[1]))
+            o.index_add_or_update(i, a)
+        for i, (s, a, want) in enumerate(configs):
+            got = h.neighbours_in_radius(P.PROBE_RADIUS, (s[0], s[1]))
+            assert got == [int(v) for v in o.query_radius(P.PROBE_RADIUS, s)], (cell, i)
+            assert got in ([], [i]), (cell, i)
+            near = _norm((a[0] - s[0], a[1] - s[1])) < P.PROBE_RADIUS
+            assert (got == [i]) == near, (cell, i)  # never within 0.4 m and outside the stencil
+            if want is not None:
+                assert near == want, i
+                continue
+            blocked_edge += near
+            free_edge += not near
+            lo = [math.floor(((s[k] - P.PROBE_RADIUS) - off[k]) / cell) for k in (0, 1)]
+            hi = [math.floor(((s[k] + P.PROBE_RADIUS) - off[k]) / cell) for k in (0, 1)]
+            col = [_Hash2D._as_usize((a[k] - off[k]) / cell) for k in (0, 1)]
+            edge_column += near and any(col[k] in (lo[k], hi[k]) and lo[k] != hi[k] for k in (0, 1))
+    # both outcomes at the stencil edges, and blocking agents that sit in the stencil's first or last column
+    assert blocked_edge > 50 and free_edge > 50 and edge_column > 50
+
+
+def test_sink_threshold_agrees_with_the_independent_restatement():
+    """The waypoint / sink test `norm(position - waypoint) < radius_sink` on the old position (lib.rs:305-336) at
+    T(r) - 1 ulp, T and T + 1 ulp from the waypoint, r = 0.3, 0.6, 1.1 (r*r inexact), 0.5 and 2.0 (exact): agents are
+    spawned at those points by source sinks that do not move them; the oracle advances, removes or wraps exactly the
+    agents the plain-Python norm puts inside."""
+    import oracle_ffi as O
+    import parity as P
+
+    configs = P.sink_threshold_configs()
+    o = O.OracleSim(400.0, 400.0, 2.0, (0.0, -200.0))
+    hl, lp = o.hl_constant((0.0, 0.0)), o.lp_none()
+    kinds = ("advance", "remove", "wrap")
+    for kind in kinds:
+        for r, wp, a, _ in configs:
+            wps = {"advance": [wp, (wp[0], 25.0)], "remove": [wp], "wrap": [a, wp]}[kind]
+            o.add_source_sink(a, r, 1.0, hl, lp, wps, kind == "wrap", 1.0)
+    o.step(1, 0)  # every source spawns; wrap agents advance to their waypoint 1 (they sit on waypoint 0)
+    _, _, d1 = o.poll_events()
+    o.step(1, 0)  # wrap agents are tested against wp; the three sources of a point are blocked by agents on it
+    s, _, d2 = o.poll_events()
+    st = o.read_state()
+    wp_of = dict(zip(st["id"].tolist(), st["next_waypoint"].tolist()))
+    n = len(configs)
+    inside = [_norm((a[0] - wp[0], a[1] - wp[1])) < r for r, wp, a, _ in configs]
+    assert inside == [want for _, _, _, want in configs]
+    assert [wp_of[i] for i in range(n)] == [1 if v else 0 for v in inside]                        # advance
+    assert sorted(d1.tolist()) == [n + i for i in range(n) if inside[i]]                           # remove
+    assert [wp_of[2 * n + i] for i in range(n)] == [0 if v else 1 for v in inside]                 # wrap
+    assert len(s) == 0 and len(d2) == 0 and sum(inside) == 10
