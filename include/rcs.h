@@ -174,9 +174,12 @@ int rcs_step_stats(rcs_sim* sim, rcs_stats* out);
 /* Study mode (SURVEY.md 8f-4): one step under the reference's IN-LOOP index semantic -- the index is updated inside
  * the per-agent loop (lib.rs:299), so agent i finds every agent that came earlier in the iteration order at its NEW
  * position and every later one at its old position, while the planner is handed their old states (lib.rs:281-286).
- * `order` = the iteration order as agent ids (the reference's is HashMap-random; ids missing from it come last, by
- * id); n_order == 0: ascending id.  Computed as a fixed-point iteration of whole-crowd sweeps (rcs_inloop.cuh) that
- * ends with exactly the sequential loop's result; *out_sweeps = sweeps used, max_sweeps == 0: no limit.
+ * `order` = the iteration order as agent ids (the reference's is HashMap-random); n_order == 0: ascending id.  Ids
+ * that are not live are ignored, live ids missing from the order come after it in ascending id, and an order that
+ * repeats an id is refused with RCS_ERR_ARG before anything runs.  Computed as a fixed-point iteration of whole-crowd
+ * sweeps (rcs_inloop.cuh) that ends with exactly the sequential loop's result; *out_sweeps = sweeps used,
+ * max_sweeps == 0: no limit.  Sweep 0 has no previous sweep to agree with, so max_sweeps == 1 always fails; a step
+ * that finds no fixed point within max_sweeps returns RCS_ERR_ARG, commits nothing and drops the trace.
  * Synchronous; one handle without strips, source sinks or route followers.  Same error behaviour as rcs_step. */
 int rcs_step_in_loop(rcs_sim* sim, uint64_t secs, uint32_t nanos, const uint64_t* order, uint64_t n_order,
                      uint32_t max_sweeps, uint32_t* out_sweeps);
@@ -216,7 +219,10 @@ int rcs_index_remove(rcs_sim* sim, uint64_t n, const uint64_t* ids);
 int rcs_query_radius(rcs_sim* sim, uint64_t nq, const double* qxy, const double* radius, uint64_t* offsets,
                      uint64_t* out_ids, uint64_t ids_cap);
 /* SpatialIndex::get_nearest_neighbours for nq queries (location_hash_2d.rs:151-238), including its
- * ring-search quirks; out_ids has nq*k slots, out_counts[q] <= k valid entries per query. */
+ * ring-search quirks; out_ids has nq*k slots, out_counts[q] <= k valid entries per query.  Where the
+ * reference's sort panics -- a query collects >= 2 candidates and one distance is NaN (a NaN query point,
+ * or an agent at a NaN position in cell 0) -- the whole call returns RCS_ERR_ARG ("get_nearest_neighbours:
+ * NaN distance") and writes neither out_ids nor out_counts. */
 int rcs_query_knn(rcs_sim* sim, uint64_t nq, const double* qxy, uint64_t k, uint64_t* out_ids,
                   uint64_t* out_counts);
 

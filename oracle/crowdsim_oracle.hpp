@@ -30,6 +30,7 @@
 #include <memory>
 #include <mutex>
 #include <optional>
+#include <stdexcept>
 #include <string>
 #include <unordered_map>
 #include <unordered_set>
@@ -213,9 +214,19 @@ class LocationHash2D : public SpatialIndex {
 
   // location_hash_2d.rs:151-238.  Ring search with half-open side ranges (the
   // (x-s,y-s) corner is visited twice, the (x+s,y+s) corner never), stops at the
-  // first ring that reaches n candidates, stable sort by distance.
+  // first ring that reaches n candidates, stable sort by distance.  The side bounds
+  // wrap as in release-mode Rust (a saturated query cell empties the sides whose
+  // upper bound wrapped) and the visits made are counted, so a ring whose visits
+  // were all out of bounds -- or that made none -- ends the walk.  The reference
+  // sorts with partial_cmp(..).unwrap(), which panics on a NaN distance as soon as
+  // two candidates are compared: that is NanDistance here.
+  struct NanDistance : std::domain_error {
+    NanDistance() : std::domain_error("get_nearest_neighbours: NaN distance") {}
+  };
   std::vector<AgentId> get_nearest_neighbours(uint64_t n, Vec2 position) const override {
     auto [x_idx, y_idx] = location_to_xy_signed_idx(position);
+    auto wadd = [](int64_t a, int64_t b) { return static_cast<int64_t>(static_cast<uint64_t>(a) + static_cast<uint64_t>(b)); };
+    auto wsub = [](int64_t a, int64_t b) { return static_cast<int64_t>(static_cast<uint64_t>(a) - static_cast<uint64_t>(b)); };
     std::vector<AgentId> agents;
     bool all_out_of_bounds = false;
     int64_t step = 0;
@@ -234,26 +245,26 @@ class LocationHash2D : public SpatialIndex {
       if (step == 0) {
         visit(x_idx, y_idx, num_out_of_bounds, num_scanned_cells);
       } else {
-        for (int64_t i = x_idx - step; i < x_idx + step; ++i)  // top line
-          visit(i, y_idx + step, num_out_of_bounds, num_scanned_cells);
-        for (int64_t i = x_idx - step; i < x_idx + step; ++i)  // bottom line
-          visit(i, y_idx - step, num_out_of_bounds, num_scanned_cells);
-        for (int64_t i = y_idx - step; i < y_idx + step; ++i)  // left line
-          visit(x_idx - step, i, num_out_of_bounds, num_scanned_cells);
-        for (int64_t i = y_idx - step; i < y_idx + step; ++i)  // right line
-          visit(x_idx + step, i, num_out_of_bounds, num_scanned_cells);
+        const int64_t xl = wsub(x_idx, step), xh = wadd(x_idx, step);
+        const int64_t yl = wsub(y_idx, step), yh = wadd(y_idx, step);
+        for (int64_t i = xl; i < xh; ++i) visit(i, yh, num_out_of_bounds, num_scanned_cells);  // top line
+        for (int64_t i = xl; i < xh; ++i) visit(i, yl, num_out_of_bounds, num_scanned_cells);  // bottom line
+        for (int64_t i = yl; i < yh; ++i) visit(xl, i, num_out_of_bounds, num_scanned_cells);  // left line
+        for (int64_t i = yl; i < yh; ++i) visit(xh, i, num_out_of_bounds, num_scanned_cells);  // right line
       }
       if (num_out_of_bounds == num_scanned_cells) all_out_of_bounds = true;
       step += 1;
     }
-    std::stable_sort(agents_in_ring.begin(), agents_in_ring.end(),
-                     [&](const auto& a, const auto& b) {
-                       double a_dist = norm(a.first - position);
-                       double b_dist = norm(b.first - position);
-                       return a_dist < b_dist;
-                     });
-    for (uint64_t i = 0; i < std::min<uint64_t>(n, agents_in_ring.size()); ++i)
-      agents.push_back(agents_in_ring[i].second);
+    std::vector<double> dist(agents_in_ring.size());
+    std::vector<size_t> perm(agents_in_ring.size());
+    for (size_t i = 0; i < agents_in_ring.size(); ++i) {
+      dist[i] = norm(agents_in_ring[i].first - position);
+      perm[i] = i;
+      if (std::isnan(dist[i]) && agents_in_ring.size() >= 2) throw NanDistance();
+    }
+    std::stable_sort(perm.begin(), perm.end(), [&](size_t a, size_t b) { return dist[a] < dist[b]; });
+    for (uint64_t i = 0; i < std::min<uint64_t>(n, perm.size()); ++i)
+      agents.push_back(agents_in_ring[perm[i]].second);
     return agents;
   }
 
@@ -704,6 +715,11 @@ class Simulation {
 
   // lib.rs:195-383
   Status step(Duration dur) {
+    if (iter_order_ == IterOrder::Custom) {  // the reference visits every agent once: a repeated id is refused
+      std::unordered_set<AgentId> seen;
+      for (AgentId id : custom_order_)
+        if (!seen.insert(id).second) return Status::Err("an id occurs twice in the order");
+    }
     // --- A. spawn phase, lib.rs:199-254.  All probes run before any insertion.
     struct ToAdd {
       uint64_t id;
@@ -861,8 +877,15 @@ class Simulation {
   std::vector<AgentId> iteration_order() const {
     std::vector<AgentId> order;
     if (iter_order_ == IterOrder::Custom) {
+      // ids that are not live are ignored; live ids missing from the order come last, in ascending id
+      std::unordered_set<AgentId> listed(custom_order_.begin(), custom_order_.end());
       for (AgentId id : custom_order_)
         if (agents.count(id)) order.push_back(id);
+      std::vector<AgentId> rest;
+      for (const auto& kv : agents)
+        if (!listed.count(kv.first)) rest.push_back(kv.first);
+      std::sort(rest.begin(), rest.end());
+      order.insert(order.end(), rest.begin(), rest.end());
       return order;
     }
     order.reserve(agents.size());

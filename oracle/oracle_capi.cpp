@@ -260,8 +260,16 @@ uint64_t orc_query_radius(void* h, double radius, double x, double y, uint64_t* 
   for (uint64_t i = 0; i < std::min<uint64_t>(cap, v.size()); ++i) out[i] = v[i];
   return v.size();
 }
+// UINT64_MAX (and orc_last_error) where the reference panics: a NaN distance among >= 2 candidates
 uint64_t orc_query_knn(void* h, uint64_t n, double x, double y, uint64_t* out, uint64_t cap) {
-  auto v = static_cast<OrcSim*>(h)->index->get_nearest_neighbours(n, {x, y});
+  auto* s = static_cast<OrcSim*>(h);
+  std::vector<AgentId> v;
+  try {
+    v = s->index->get_nearest_neighbours(n, {x, y});
+  } catch (const LocationHash2D::NanDistance& e) {
+    s->last_error = e.what();
+    return ~0ull;
+  }
   for (uint64_t i = 0; i < std::min<uint64_t>(cap, v.size()); ++i) out[i] = v[i];
   return v.size();
 }

@@ -1151,14 +1151,30 @@ __global__ void query_radius_kernel(GridDev g, const uint32_t* __restrict__ cell
 // and cell (x+s, y+s) never; the walk stops after the first ring that brings the candidate count to n
 // (not a true kNN); candidates are then STABLY sorted by distance (sort_by + partial_cmp, :226-230).
 // f(c) is called for every valid data cell in visiting order and returns the number of agents in it.
+//
+// The side bounds x_idx +- step and y_idx +- step wrap in two's complement, as release-mode Rust computes them: a
+// saturated query cell (x = +inf, or >= 2^63 cells away) leaves the sides whose upper bound wrapped EMPTY.  So the
+// visits are counted, not assumed to be 8*step, and a ring whose visits were all out of bounds ends the walk, an empty
+// ring included.  Termination: counting the visits makes this walk the reference's, ring for ring.  Away from
+// saturation a ring at Chebyshev distance step eventually has every cell at a negative coordinate or past the data;
+// for a saturated x the only side that can reach the grid is the column x_idx - step, whose wrapped data index drops
+// by nx per step while its row window grows by one, so it leaves [0, len).  A side loop runs at most 2*step times
+// (i < hi, so i + 1 never overflows).
 // ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ int64_t wrapping_add_i64(int64_t a, int64_t b) {
+  return (int64_t)((uint64_t)a + (uint64_t)b);
+}
+__device__ __forceinline__ int64_t wrapping_sub_i64(int64_t a, int64_t b) {
+  return (int64_t)((uint64_t)a - (uint64_t)b);
+}
+
 template <class F>
 __device__ __forceinline__ uint64_t knn_walk(const GridDev& g, double px, double py, uint64_t n, F&& f) {
   const int64_t x_idx = f64_floor_as_i64(div_floor(px - g.offx, g));  // location_to_xy_signed_idx, :68-72
   const int64_t y_idx = f64_floor_as_i64(div_floor(py - g.offy, g));
   uint64_t have = 0;
   bool all_oob = false;
-  auto visit = [&](int64_t cx, int64_t cy, uint64_t& oob) {
+  auto visit = [&](int64_t cx, int64_t cy, uint64_t& oob, uint64_t& scanned) {
     // signed_idx_to_data_idx, :74-85
     bool ok = cx >= 0 && cy >= 0;
     uint64_t idx = 0;
@@ -1168,18 +1184,19 @@ __device__ __forceinline__ uint64_t knn_walk(const GridDev& g, double px, double
     }
     if (ok) have += f(idx);
     else oob += 1;
+    scanned += 1;
   };
   for (int64_t step = 0; have < n && !all_oob; ++step) {
     uint64_t oob = 0, scanned = 0;
     if (step == 0) {
-      visit(x_idx, y_idx, oob);
-      scanned = 1;
+      visit(x_idx, y_idx, oob, scanned);
     } else {
-      for (int64_t i = x_idx - step; i < x_idx + step; ++i) visit(i, y_idx + step, oob);  // top line
-      for (int64_t i = x_idx - step; i < x_idx + step; ++i) visit(i, y_idx - step, oob);  // bottom line
-      for (int64_t i = y_idx - step; i < y_idx + step; ++i) visit(x_idx - step, i, oob);  // left line
-      for (int64_t i = y_idx - step; i < y_idx + step; ++i) visit(x_idx + step, i, oob);  // right line
-      scanned = (uint64_t)(8 * step);
+      const int64_t xl = wrapping_sub_i64(x_idx, step), xh = wrapping_add_i64(x_idx, step);
+      const int64_t yl = wrapping_sub_i64(y_idx, step), yh = wrapping_add_i64(y_idx, step);
+      for (int64_t i = xl; i < xh; ++i) visit(i, yh, oob, scanned);  // top line
+      for (int64_t i = xl; i < xh; ++i) visit(i, yl, oob, scanned);  // bottom line
+      for (int64_t i = yl; i < yh; ++i) visit(xl, i, oob, scanned);  // left line
+      for (int64_t i = yl; i < yh; ++i) visit(xh, i, oob, scanned);  // right line
     }
     if (oob == scanned) all_oob = true;
   }
@@ -1218,17 +1235,20 @@ __global__ void knn_fill_kernel(GridDev g, const uint32_t* __restrict__ cell_sta
   });
 }
 
-// pass 2: one warp per query; stable rank by distance, the first min(k, m) go out
+// pass 2: one warp per query; stable rank by distance, the first min(k, m) go out.  The rank is a permutation only
+// under a total order: a NaN distance among >= 2 candidates is where the reference's partial_cmp(..).unwrap() panics
+// (:226-230), so it sets *nan_flag instead and the host refuses the whole call.
 __global__ void knn_select_kernel(uint32_t nq, uint64_t k, const uint32_t* __restrict__ offsets,
                                   const uint32_t* __restrict__ cand_slot, const double* __restrict__ cand_dist,
                                   const uint64_t* __restrict__ ids, uint64_t* __restrict__ out_ids,
-                                  uint64_t* __restrict__ out_counts) {
+                                  uint64_t* __restrict__ out_counts, uint32_t* __restrict__ nan_flag) {
   const uint32_t q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const uint32_t lane = threadIdx.x & 31u;
   if (q >= nq) return;
   const uint32_t s = offsets[q], m = offsets[q + 1] - s;
   for (uint32_t t = lane; t < m; t += 32) {
     const double d = cand_dist[s + t];
+    if (d != d && m >= 2) *nan_flag = 1u;
     uint32_t rank = 0;
     for (uint32_t u = 0; u < m; ++u) {
       const double du = cand_dist[s + u];

@@ -278,6 +278,8 @@ class LocationHash2D:
         return [int(v) for v in ids[0, : int(counts[0])]]
 
     def query_knn(self, qxy: np.ndarray, k: int) -> Tuple[np.ndarray, np.ndarray]:
+        """Batched get_nearest_neighbours: ids[nq, max(k, 1)] and counts[nq].  Raises CrowdsimError where the
+        reference's sort panics: a query with >= 2 candidates of which one is at a NaN distance."""
         qxy = _f64(qxy).reshape(-1, 2)
         nq = qxy.shape[0]
         ids = np.zeros((nq, max(k, 1)), dtype=np.uint64)
@@ -424,7 +426,11 @@ class Simulation:
 
     def step_in_loop(self, dur: Duration, order=None, max_sweeps: int = 0) -> int:
         """One step under the reference's in-loop index semantic (lib.rs:299; SURVEY.md 8f-4) for the iteration order
-        `order` (agent ids; None = ascending id).  Returns the number of whole-crowd sweeps the fixed point took."""
+        `order` (agent ids; None = ascending id).  Ids that are not live are ignored; live agents missing from `order`
+        are visited after it in ascending id; an order that repeats an id raises CrowdsimError and changes nothing.
+        max_sweeps = 0: no limit; otherwise a step without a fixed point within max_sweeps raises and commits nothing
+        (max_sweeps = 1 always does: sweep 0 has nothing to agree with).  Returns the number of whole-crowd sweeps
+        the fixed point took."""
         if self._host_hl:
             self._run_host_planners()
         sweeps = C.c_uint32()

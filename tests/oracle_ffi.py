@@ -244,6 +244,8 @@ class OracleSim:
     def query_knn(self, n, p, cap=1 << 16):
         out = np.zeros(cap, dtype=np.uint64)
         m = self.L.orc_query_knn(self.h, int(n), float(p[0]), float(p[1]), _p(out, u64p), cap)
+        if m == 2**64 - 1:
+            raise OracleError(1, self.L.orc_last_error(self.h).decode())
         return out[: int(m)].copy()
 
 

@@ -123,8 +123,12 @@ def _same(ta, tb, keys):
         assert a.shape == b.shape and len(bad) == 0, (k, [(int(i), hex(int(a[i])), hex(int(b[i]))) for i in bad[:8]])
 
 
-def build_oracle(scene: SC.Scene, index_mode=O.DEFERRED, inject_velocity=True) -> O.OracleSim:
-    o = O.OracleSim(scene.width, scene.height, scene.cell, scene.offset, index_mode=index_mode)
+def build_oracle(scene: SC.Scene, index_mode=O.DEFERRED, inject_velocity=True, order=None) -> O.OracleSim:
+    """order: the iteration order as agent ids (the oracle's Custom order); None = ascending id."""
+    o = O.OracleSim(scene.width, scene.height, scene.cell, scene.offset, index_mode=index_mode,
+                    iter_order=O.ASCENDING_ID if order is None else O.CUSTOM)
+    if order is not None:
+        o.set_custom_order(order)
     kind, v = scene.hl
     hl = o.hl_parity(v) if kind == "parity" else o.hl_constant(v)
     lp = o.lp_none() if scene.lp[0] == "none" else o.lp_zanlungo(*scene.lp[1:])
@@ -201,3 +205,50 @@ def resync(g, o) -> None:
     so = o.read_state()
     if len(so["id"]):
         g.set_state(None, so["x"], so["y"], so["vx"], so["vy"])
+
+
+def _cell_centres(cells, nx, cell=1.0):
+    """Insertable points at the centre of data cells (x = idx // nx, y = idx % nx: the index formula's own inverse)."""
+    return np.array([[(c // nx + 0.5) * cell, (c % nx + 0.5) * cell] for c in cells], dtype=np.float64)
+
+
+def saturated_knn_cases():
+    """(name, (width, height, cell, offset), agents, query, k) for the kNN ring walk at a saturated query cell.
+    x = +inf floors to x_idx = i64::MAX; with an even nx, MAX * nx wraps to -nx, so a row y_idx in [nx, nx + len)
+    lands inside the grid and the walk goes on; from ring 1 the sides whose upper bound wraps are empty.  With an odd
+    nx the same query is outside at ring 0.  x = (2^63 - 1024) cells on a row 1024 * nx up hits the data through the
+    wrapped index in every ring until its bounds wrap at ring 1024, which is then all outside."""
+    even = (8.0, 8.0, 1.0, (0.0, 0.0))
+    odd = (9.0, 9.0, 1.0, (0.0, 0.0))
+    wide = (64.0, 4.0, 1.0, (0.0, 0.0))  # nx = 64, ny = 4: rows >= 4 alias into the next columns
+    a_even = _cell_centres([12, 3, 4, 45, 63], 8)
+    a_odd = _cell_centres([12, 3, 4, 45, 80], 9)
+    a_wide = _cell_centres([100, 37, 200, 5, 255], 64)
+    far = 2.0 ** 63 - 1024.0
+    return [
+        ("inf_even", even, a_even, (INF, 20.5), 10),     # ring 0: data cell 20 - 8 = 12; ring 1: cells 3, 4
+        ("inf_even_k1", even, a_even, (INF, 20.5), 1),
+        ("inf_even_row", even, a_even, (INF, 71.5), 10),  # the last aliased row: data cell 63
+        ("inf_odd", odd, a_odd, (INF, 20.5), 10),
+        ("inf_inf", even, a_even, (INF, INF), 10),
+        ("minus_inf", even, a_even, (-INF, 3.5), 10),
+        ("y_inf", even, a_even, (3.5, INF), 10),
+        ("far_x", wide, a_wide, (far, 1024.0 * 64 + 100.5), 4000),
+        ("far_x_k3", wide, a_wide, (far, 1024.0 * 64 + 100.5), 3),
+    ]
+
+
+# kNN around NaN distances on an 8 x 8 grid of 1 m cells at the origin: (agents with id = row, query, k, error?).
+# The reference's sort panics on a NaN distance once two candidates are compared; a single candidate is returned.
+NAN_KNN_CASES = [
+    ([(NAN, NAN), (0.5, 0.5), (3.5, 3.5)], (0.2, 0.3), 1, True),    # cell 0 holds two, one NaN: k = 1 is enough
+    ([(NAN, NAN), (0.5, 0.5), (3.5, 3.5)], (3.5, 3.6), 1, False),   # the walk stops before cell 0
+    ([(NAN, NAN), (0.5, 0.5), (3.5, 3.5)], (3.5, 3.6), 3, True),
+    ([(NAN, 2.0), (0.5, 0.5)], (6.5, 6.5), 9, True),                  # NaN x only
+    ([(NAN, NAN)], (0.5, 0.5), 5, False),                             # one candidate: no comparison
+    ([(NAN, NAN)], (1.5, 1.5), 5, True),                              # cell 0 is ring 1's doubled corner
+    ([(0.5, 0.5), (3.5, 3.5)], (NAN, NAN), 1, False),                 # NaN query, one candidate in cell 0
+    ([(0.5, 0.5), (3.5, 3.5)], (NAN, NAN), 2, True),
+    ([(0.5, 0.5), (3.5, 3.5)], (NAN, 3.5), 1, True),                  # column 0, row 3: ring 3 brings both
+    ([(0.5, 0.5), (3.5, 3.5)], (NAN, NAN), 0, False),
+]

@@ -418,20 +418,42 @@ def test_radius_query_agrees_with_the_independent_hash_grid():
         assert lst == [int(j) for j in nb[off[i]:off[i + 1]]], i
 
 
-def _nearest(h, n, p):
+_I64_MIN, _I64_MAX = -(1 << 63), (1 << 63) - 1
+
+
+def _floor_i64(v):
+    """`f64.floor() as i64`: saturating, NaN -> 0 (math.floor raises on inf and NaN)."""
+    if v != v:
+        return 0
+    if v >= 2.0 ** 63:
+        return _I64_MAX
+    if v <= -(2.0 ** 63):
+        return _I64_MIN
+    return math.floor(v)
+
+
+def _wrap_i64(v):
+    """Two's-complement wrap of an exact integer, as release-mode Rust's i64 `+` and `-`."""
+    return (v + (1 << 63)) % (1 << 64) - (1 << 63)
+
+
+def _nearest(h, n, p, stats=None):
     """get_nearest_neighbours (location_hash_2d.rs:151-238), second restatement: rings of cells around the query cell
     with HALF-OPEN sides (the (x-s, y-s) corner is visited twice, the (x+s, y+s) corner never), stop at the first ring
-    that brings the candidate count to n or when a whole ring is outside the grid, then a stable sort by distance."""
-    x_idx = math.floor((p[0] - h.off[0]) / h.res)
-    y_idx = math.floor((p[1] - h.off[1]) / h.res)
+    that brings the candidate count to n or whose visits were all outside the grid, then a stable sort by distance.
+    Release-mode Rust arithmetic: the query cell saturates to i64, the side bounds x_idx +- step wrap (a side whose
+    upper bound wrapped is empty) and so does the data index cx * nx + cy (u64).  A NaN distance among >= 2 candidates
+    raises, where the reference's partial_cmp(..).unwrap() panics.  `stats["rings"]`: the rings walked."""
+    x_idx = _floor_i64((p[0] - h.off[0]) / h.res)
+    y_idx = _floor_i64((p[1] - h.off[1]) / h.res)
     ring = []
 
     def visit(cx, cy, stat):
         stat[1] += 1
-        if cx < 0 or cy < 0 or cx * h.nx + cy >= h.len:
+        if cx < 0 or cy < 0 or (cx * h.nx + cy) % (1 << 64) >= h.len:
             stat[0] += 1
             return
-        for j in sorted(h.cells.get(cx * h.nx + cy, ())):
+        for j in sorted(h.cells.get((cx * h.nx + cy) % (1 << 64), ())):
             ring.append((h.loc[j], j))
 
     step, all_out = 0, False
@@ -440,18 +462,25 @@ def _nearest(h, n, p):
         if step == 0:
             visit(x_idx, y_idx, stat)
         else:
-            for i in range(x_idx - step, x_idx + step):
-                visit(i, y_idx + step, stat)
-            for i in range(x_idx - step, x_idx + step):
-                visit(i, y_idx - step, stat)
-            for i in range(y_idx - step, y_idx + step):
-                visit(x_idx - step, i, stat)
-            for i in range(y_idx - step, y_idx + step):
-                visit(x_idx + step, i, stat)
+            xl, xh = _wrap_i64(x_idx - step), _wrap_i64(x_idx + step)
+            yl, yh = _wrap_i64(y_idx - step), _wrap_i64(y_idx + step)
+            for i in range(xl, xh):
+                visit(i, yh, stat)
+            for i in range(xl, xh):
+                visit(i, yl, stat)
+            for i in range(yl, yh):
+                visit(xl, i, stat)
+            for i in range(yl, yh):
+                visit(xh, i, stat)
         all_out = stat[0] == stat[1]
         step += 1
-    ring.sort(key=lambda e: _norm((e[0][0] - p[0], e[0][1] - p[1])))  # list.sort is stable, like the reference's
-    return [j for _, j in ring[:n]]
+    if stats is not None:
+        stats["rings"] = step
+    dist = [_norm((e[0][0] - p[0], e[0][1] - p[1])) for e in ring]
+    if len(ring) >= 2 and any(d != d for d in dist):
+        raise ValueError("get_nearest_neighbours: NaN distance")
+    order = sorted(range(len(ring)), key=lambda k: dist[k])  # sorted is stable, like the reference's sort_by
+    return [ring[k][1] for k in order[:n]]
 
 
 def test_nearest_neighbours_agree_with_the_independent_hash_grid():
@@ -469,6 +498,118 @@ def test_nearest_neighbours_agree_with_the_independent_hash_grid():
         assert _nearest(h, 4, (q[0], q[1])) == want, (k, q)
         lo, hi = int(g["rad_offsets"][k]), int(g["rad_offsets"][k + 1])
         assert h.neighbours_in_radius(float(g["radius"][0]), (q[0], q[1])) == [int(v) for v in g["rad_ids"][lo:hi]]
+
+
+def _knn_pair(w, h, cell, off, pts):
+    """The oracle's index and the second hash grid holding the same agents (id = row)."""
+    import oracle_ffi as O
+
+    o, hh = O.OracleSim(w, h, cell, off), _Hash2D(w, h, cell, off)
+    for i, p in enumerate(pts):
+        o.index_add_or_update(i, p)
+        hh.add_or_update(i, (float(p[0]), float(p[1])))
+    return o, hh
+
+
+def test_nan_distance_in_the_nearest_neighbour_sort_is_an_error():
+    """The reference sorts the candidates with partial_cmp(..).unwrap() (location_hash_2d.rs:226-230): a NaN distance
+    panics as soon as two candidates are compared.  Both restatements raise there and return a single candidate as is:
+    an agent at a NaN position (filed in cell 0 by the saturating cast) next to a finite one in cell 0, a NaN query (its
+    cell floors to (0, 0)), the lone NaN agent, and a query whose ring visits the NaN agent's cell twice (the doubled
+    (x-s, y-s) corner)."""
+    import oracle_ffi as O
+
+    import parity as P
+
+    for agents, q, k, err in P.NAN_KNN_CASES:
+        o, hh = _knn_pair(8.0, 8.0, 1.0, (0.0, 0.0), np.array(agents))
+        if err:
+            try:
+                _nearest(hh, k, q)
+                raise AssertionError((agents, q, k))
+            except ValueError as e:
+                assert str(e) == "get_nearest_neighbours: NaN distance"
+            try:
+                o.query_knn(k, q)
+                raise AssertionError((agents, q, k))
+            except O.OracleError as e:
+                assert str(e) == "get_nearest_neighbours: NaN distance"
+        else:
+            assert list(o.query_knn(k, q)) == _nearest(hh, k, q), (agents, q, k)
+    o, hh = _knn_pair(8.0, 8.0, 1.0, (0.0, 0.0), np.array([(NAN, NAN)]))
+    assert _nearest(hh, 5, (0.5, 0.5)) == [0]
+    o, hh = _knn_pair(8.0, 8.0, 1.0, (0.0, 0.0), np.array([(0.5, 0.5), (3.5, 3.5)]))
+    assert _nearest(hh, 1, (NAN, NAN)) == [0]
+
+
+def test_ring_walk_at_a_saturated_query_cell_agrees_with_the_independent_hash_grid():
+    """The ring walk where release-mode Rust wraps: the query cell saturates to i64::MAX (x = +inf) or sits 2^63 - 1024
+    cells out, the side bounds x_idx + step wrap and empty their sides, and the walk ends at the first ring whose
+    visits were all outside the grid (tests/parity.py saturated_knn_cases).  Both restatements agree, and each case's
+    class is hit: the even-nx +inf query finds agents through the wrapped index, the odd-nx one nothing, and the far
+    query walks all 1025 rings, collecting agents many times over."""
+    import parity as P
+
+    got = {}
+    for name, (w, h, cell, off), pts, q, k in P.saturated_knn_cases():
+        o, hh = _knn_pair(w, h, cell, off, pts)
+        st = {}
+        want = _nearest(hh, k, q, st)
+        assert list(o.query_knn(k, q)) == want, name
+        got[name] = (want, st["rings"])
+    assert got["inf_even"] == ([0, 1, 2], 3)  # cell 12 at ring 0, cells 3 and 4 on ring 1's left side; ring 2 is out
+    assert got["inf_even_k1"] == ([0], 1)
+    assert got["inf_even_row"][0][0] == 4 and got["inf_even_row"][1] > 3  # the left side stays in the data longer
+    assert got["inf_odd"] == ([], 1) and got["inf_inf"] == ([], 1) and got["minus_inf"] == ([], 1)
+    assert got["y_inf"] == ([], 1)
+    far, rings = got["far_x"]
+    assert rings == 1025 and len(far) > 5 * 10 and set(far) == set(range(5))
+    assert got["far_x_k3"][0] == far[:3]
+
+
+def test_in_loop_custom_order_appends_missing_agents_and_refuses_a_repeated_id():
+    """The oracle's Custom iteration order (the in-loop study mode's): ids that are not live are ignored, live ids
+    missing from the order are visited after it in ascending id (the reference visits every agent, lib.rs:259), and
+    an order that repeats an id is refused before anything moves."""
+    import oracle_ffi as O
+    import parity as P
+    from rmf_crowdsim_b200 import scenes as SC
+
+    rng = np.random.default_rng(5)
+    scene = SC.uniform_crowd(10, "shuffled", cell=1.0, eyesight=2.5, margin=8.0, seed=13,
+                             lp=("zanlungo", 0.05, 1.0, 0.0, 0.5, 200.0, 0.1))
+    scene.vxy = scene.vxy + rng.uniform(-0.3, 0.3, size=scene.vxy.shape)
+    perm = rng.permutation(scene.n).astype(np.uint64)
+    part = perm[:60]
+    full = np.concatenate([part, np.sort(perm[60:])])
+    gone = int(perm[-1])  # removed below
+    noisy = np.concatenate([[1000, gone], part[:30], [2 ** 40], part[30:]]).astype(np.uint64)
+    runs = {}
+    for name, order in (("partial", part), ("full", full), ("noisy", noisy)):
+        o = P.build_oracle(scene, index_mode=O.IN_LOOP, order=order)
+        o.remove_agent(gone)
+        o.enable_trace(True)
+        for _ in range(2):
+            o.step(0, 250_000_000)
+        runs[name] = (o.read_state(), o.read_trace())
+    want = P.build_oracle(scene, index_mode=O.IN_LOOP, order=full[full != gone])
+    want.remove_agent(gone)
+    want.enable_trace(True)
+    for _ in range(2):
+        want.step(0, 250_000_000)
+    ws, wt = want.read_state(), want.read_trace()
+    assert len(wt["id"]) == scene.n - 1  # every live agent was visited
+    for name, (st, tr) in runs.items():
+        P._same(st, ws, ("id", "x", "y", "vx", "vy"))
+        P._same(tr, wt, ("id", "t_i", "fx", "fy", "nb_offsets", "nb_ids"))
+    o = P.build_oracle(scene, index_mode=O.IN_LOOP, order=np.array([3, 1, 3], dtype=np.uint64))
+    before = o.read_state()
+    try:
+        o.step(0, 250_000_000)
+        raise AssertionError("a repeated id was accepted")
+    except O.OracleError as e:
+        assert str(e) == "an id occurs twice in the order"
+    P._same(o.read_state(), before, ("id", "x", "y", "vx", "vy"))
 
 
 def test_source_sink_stream_agrees_with_the_independent_restatement():
