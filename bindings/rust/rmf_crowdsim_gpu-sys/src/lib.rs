@@ -80,6 +80,10 @@ extern "C" {
     pub fn rcs_hl_none(sim: *mut rcs_sim, out_hl: *mut u32) -> c_int;
     pub fn rcs_hl_route(sim: *mut rcs_sim, n_points: u64, xy: *const f64, out_hl: *mut u32) -> c_int;
     pub fn rcs_hl_route_set_target(sim: *mut rcs_sim, n: u64, ids: *const u64) -> c_int;
+    pub fn rcs_hl_route_table(sim: *mut rcs_sim, n_legs: u64, targets_xy: *const f64, leg_points: *const u64,
+                              xy: *const f64, out_hl: *mut u32) -> c_int;
+    pub fn rcs_hl_route_table_set_target(sim: *mut rcs_sim, hl: u32, n: u64, ids: *const u64,
+                                         targets_xy: *const f64) -> c_int;
 
     pub fn rcs_add_agents(sim: *mut rcs_sim, n: u64, xy: *const f64, hl: u32, lp: u32, eyesight: f64,
                           out_ids: *mut u64) -> c_int;

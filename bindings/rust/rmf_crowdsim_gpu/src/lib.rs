@@ -59,6 +59,10 @@ pub enum HighLevelPlan {
     None,
     /// the per-step half of `rmf::RMFPlanner` (rmf/mod.rs:197-215) on a route the host planned
     Route(Vec<Point>),
+    /// `rmf::RMFPlanner` (rmf/mod.rs:86-241) with a route cache the host filled: (target, route) legs;
+    /// `set_target(point)` selects the leg whose target equals the point.  A source sink with this planner may have
+    /// any number of waypoints, each with a leg.
+    RouteTable(Vec<(Point, Vec<Point>)>),
     /// any user planner, evaluated on the host every step
     Host(Arc<Mutex<dyn HighLevelPlanner>>),
 }
@@ -121,6 +125,15 @@ impl Simulation {
             HighLevelPlan::Route(r) => {
                 let xy: Vec<f64> = r.iter().flat_map(|p| [p.x, p.y]).collect();
                 unsafe { sys::rcs_hl_route(self.h, r.len() as u64, xy.as_ptr(), &mut out) }
+            }
+            HighLevelPlan::RouteTable(legs) => {
+                let targets: Vec<f64> = legs.iter().flat_map(|(t, _)| [t.x, t.y]).collect();
+                let counts: Vec<u64> = legs.iter().map(|(_, r)| r.len() as u64).collect();
+                let xy: Vec<f64> = legs.iter().flat_map(|(_, r)| r.iter().flat_map(|p| [p.x, p.y])).collect();
+                unsafe {
+                    sys::rcs_hl_route_table(self.h, legs.len() as u64, targets.as_ptr(), counts.as_ptr(), xy.as_ptr(),
+                                            &mut out)
+                }
             }
             HighLevelPlan::Host(_) => {
                 if let Some(hh) = self.hl_host_handle {

@@ -94,6 +94,7 @@ int rcs_lp_zanlungo(rcs_sim* sim, double agent_scale, double obstacle_scale, dou
  *  constant: Some(v) for every agent            (fixture of lib.rs:391-420)
  *  parity  : even id -> Some(-v), odd -> Some(v) (fixture of rmf_crowdsim_viz/src/main.rs:20-30)
  *  route   : rmf::RMFPlanner's waypoint follower on a caller-supplied route (see rcs_hl_route)
+ *  route table: the same follower on caller-supplied legs, one per set_target point (see rcs_hl_route_table)
  *  host    : Some(table[id]) as uploaded by rcs_set_preferred_velocity, None for ids never set
  *            (slow path that keeps user-implemented HighLevelPlanner trait objects usable)
  *  none    : always None  => velocity (0,0)     (lib.rs:263-273) */
@@ -108,9 +109,28 @@ int rcs_hl_host(rcs_sim* sim, uint32_t* out_hl);
  * point 0 through HighLevelPlanner::set_target: automatically when a SourceSink spawns them (lib.rs:242-249)
  * and whenever they reach one of its waypoints (lib.rs:326-333), or explicitly with rcs_hl_route_set_target.
  * A SourceSink with a route planner takes exactly ONE waypoint, the sink (the reference plans a new route per waypoint;
- * here a planner is one polyline): rcs_add_source_sink refuses more with RCS_ERR_ARG. */
+ * here a planner is one polyline): rcs_add_source_sink refuses more with RCS_ERR_ARG.  A source sink with
+ * intermediate waypoints takes a route-table planner (rcs_hl_route_table).  n_points: 1..65534. */
 int rcs_hl_route(rcs_sim* sim, uint64_t n_points, const double* xy, uint32_t* out_hl);
 int rcs_hl_route_set_target(rcs_sim* sim, uint64_t n, const uint64_t* ids);
+/* RMFPlanner with a route cache the caller has filled: the routes that set_target would plan, as LEGS.
+ * Leg k: target (targets_xy[2k], targets_xy[2k+1]), polyline of leg_points[k] points; the legs' points are
+ * concatenated in xy.  set_target(agent, point, tolerance) makes the leg whose target == point (IEEE equality on both
+ * coordinates; NaN never matches; the tolerance is ignored) the agent's cache entry, at its route point 0.
+ * get_desired_velocity is rcs_hl_route's follower on the current leg: it advances from point k to k+1 within 0.1 m
+ * unless k is the leg's last point.  In a SourceSink the spawn calls set_target(waypoints[0]) and every advance to
+ * waypoint k+1 calls set_target(waypoints[k+1]); a loop_forever wrap calls nothing (lib.rs:305-336), so the agent
+ * keeps its last leg.  A one-leg table whose target is the sink runs exactly as rcs_hl_route on the same polyline.
+ * RCS_ERR_ARG, nothing registered: no legs, a leg without points, two legs with equal targets, more than 65534
+ * points in all.  rcs_add_source_sink refuses (RCS_ERR_ARG, nothing added) a route-table planner with a waypoint
+ * that has no leg. */
+int rcs_hl_route_table(rcs_sim* sim, uint64_t n_legs, const double* targets_xy, const uint64_t* leg_points,
+                       const double* xy, uint32_t* out_hl);
+/* set_target(agent, targets_xy[i], ..) of planner hl for the agents ids[i] (agents added with rcs_add_agents; an id
+ * listed twice takes its last target).  An unknown id, an agent not driven by hl, a point without a leg, or an hl that
+ * is not a route-table planner -> RCS_ERR_ARG and nothing is written. */
+int rcs_hl_route_table_set_target(rcs_sim* sim, uint32_t hl, uint64_t n, const uint64_t* ids,
+                                  const double* targets_xy);
 int rcs_hl_none(rcs_sim* sim, uint32_t* out_hl);
 
 /* ---- agents ---------------------------------------------------------------------------------- */

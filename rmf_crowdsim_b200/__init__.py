@@ -15,6 +15,7 @@ from .sim import (  # noqa: F401
     NoLocalPlan,
     ParityVelocityPlan,
     RouteFollowPlan,
+    RouteTablePlan,
     Simulation,
     SourceSink,
     Zanlungo,
@@ -23,5 +24,5 @@ from .sim import (  # noqa: F401
 __all__ = [
     "Agent", "ConstantVelocityPlan", "CrowdGenerator", "CrowdsimError", "Duration", "EventListener",
     "HighLevelPlanner", "LocalPlanner", "LocationHash2D", "MonotonicCrowd", "NoHighLevelPlan", "NoLocalPlan",
-    "ParityVelocityPlan", "RouteFollowPlan", "Simulation", "SourceSink", "Zanlungo",
+    "ParityVelocityPlan", "RouteFollowPlan", "RouteTablePlan", "Simulation", "SourceSink", "Zanlungo",
 ]

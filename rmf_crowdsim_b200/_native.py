@@ -94,6 +94,8 @@ SIGNATURES = {
     "rcs_hl_host": (C.c_int, [C.c_void_p, c_u32p]),
     "rcs_hl_route": (C.c_int, [C.c_void_p, C.c_uint64, c_f64p, c_u32p]),
     "rcs_hl_route_set_target": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p]),
+    "rcs_hl_route_table": (C.c_int, [C.c_void_p, C.c_uint64, c_f64p, c_u64p, c_f64p, c_u32p]),
+    "rcs_hl_route_table_set_target": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint64, c_u64p, c_f64p]),
     "rcs_hl_none": (C.c_int, [C.c_void_p, c_u32p]),
     "rcs_add_agents": (C.c_int, [C.c_void_p, C.c_uint64, c_f64p, C.c_uint32, C.c_uint32, C.c_double, c_u64p]),
     "rcs_remove_agents": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p]),

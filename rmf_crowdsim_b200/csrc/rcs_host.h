@@ -12,8 +12,10 @@
 #include <cstdlib>
 #include <cstring>
 #include <limits>
+#include <map>
 #include <numeric>
 #include <string>
+#include <unordered_set>
 #include <vector>
 
 #include "rcs_kernels.cuh"
@@ -32,8 +34,17 @@ struct LPDesc {
 struct HLDesc {
   uint32_t kind;
   double vx, vy;
-  uint32_t route_off, route_n;  // HL_ROUTE: polyline in the route table
+  uint32_t route_off, route_n;  // HL_ROUTE / HL_ROUTE_TABLE: the planner's table in the route array
+  // HL_ROUTE_TABLE: leg target -> index of the leg's first point within the planner's table.  std::less on doubles
+  // is IEEE equality for non-NaN keys (+0 == -0); NaN targets are never inserted, so they never match.
+  std::map<std::pair<double, double>, uint32_t> legs;
 };
+// RouteTablePlan's leg lookup: the leg whose target == (x, y) on both coordinates -> its first point, or -1
+inline int64_t leg_of(const HLDesc& h, double x, double y) {
+  if (x != x || y != y) return -1;
+  const auto it = h.legs.find({x, y});
+  return it == h.legs.end() ? -1 : (int64_t)it->second;
+}
 struct GroupKey {
   uint32_t hl, lp;
   double eyesight;
@@ -161,7 +172,9 @@ struct rcs_sim {
   bool any_zanlungo = false;
   bool any_route = false;            // an HL_ROUTE group exists: steps take the sorted path (it carries `wp`)
   std::vector<double> routes;        // route table, interleaved x,y
+  std::vector<uint32_t> route_end;   // per route point: one past the last point of its leg, within its planner's table
   double* d_routes = nullptr;
+  uint32_t* d_route_end = nullptr;
   bool routes_dirty = false;
   bool have_host_hl = false;
   rcs::DevStatus* d_status = nullptr;
@@ -187,8 +200,10 @@ struct rcs_sim {
   // source sinks
   std::vector<rcs::SourceSinkDev> sources;  // index = source sink id (removed ones stay with alive = 0)
   std::vector<double> ss_wp;                // shared waypoint table, interleaved
+  std::vector<uint32_t> ss_rwp;             // per waypoint (offsets of ss_wp): route-follower entry of set_target
   rcs::SourceSinkDev* d_sources = nullptr;
   double* d_ss_wp = nullptr;
+  uint32_t* d_ss_rwp = nullptr;
   uint32_t* d_blocked = nullptr;
   // strips: spawn set of the step as a bitmap over the source ids: this rank's, every rank's (single-process
   // transport: staging for the other ranks' bitmaps), and the sum over the ranks

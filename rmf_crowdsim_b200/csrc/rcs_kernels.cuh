@@ -674,6 +674,7 @@ struct StepArgs {
   StripDev strip;
   const SourceSinkDev* ss;         // nullptr when there are no source sinks
   const double* ss_wp;             // waypoint table, interleaved x,y
+  const uint32_t* ss_rwp;          // per waypoint: the route-follower entry set_target(waypoints[k]) gives (0: none)
   uint32_t* cnt;                   // device counters (CNT_*)
   unsigned long long* ev_destroyed;  // (id, step) pairs of agents removed at sinks
   uint32_t ev_cap;
@@ -687,11 +688,13 @@ struct StepArgs {
   uint32_t* next_count;
   uint64_t cell_lo, cell_hi;       // cells this handle indexes
   const double* routes;            // HL_ROUTE polylines, interleaved x,y
+  const uint32_t* route_end;       // per route point: one past the last point of its leg, within its planner's table
   double route_thr2;               // smallest double T with sqrt(T) >= 1e-1 (rmf/mod.rs:202)
 };
 
 // next_waypoint (lib.rs:61) lives in the low half of the per-agent `wp` word; the high half is the agent's entry
-// in the route follower's agent_cache (rmf/mod.rs:86): 0 = absent, k + 1 = heading for route point k.
+// in the route follower's agent_cache (rmf/mod.rs:86): 0 = absent, k + 1 = heading for point k of the planner's
+// table (a route-table planner's legs are concatenated in it; a route planner's table is its one route).
 constexpr uint32_t WP_MASK = 0xffffu;
 constexpr int WP_ROUTE_SHIFT = 16;
 
@@ -832,13 +835,15 @@ __device__ __forceinline__ void high_level_velocity(const StepArgs& a, uint32_t 
       me.pfy = vely;
       break;
     case HL_ROUTE: {
-      // the per-step half of RMFPlanner::get_desired_velocity (rmf/mod.rs:197-215) on a caller-supplied route
+      // the per-step half of RMFPlanner::get_desired_velocity (rmf/mod.rs:197-215) on the caller-supplied route of
+      // the agent's current leg (route-table planners; a route planner is a table of one leg)
       uint32_t rw = a.in.wp[i] >> WP_ROUTE_SHIFT;
       if (rw != 0u) {  // in agent_cache
         uint32_t wid = rw - 1u;
         const double* r = a.routes + 2 * (size_t)g.route_off;
         double dx = me.px - r[2 * wid], dy = me.py - r[2 * wid + 1];
-        if (dx * dx + dy * dy < a.route_thr2 && g.route_n > wid + 1u) {  // (pos - route[wp]).norm() < 1e-1
+        // (pos - route[wp]).norm() < 1e-1 and route[wp] is not the last point of the leg
+        if (dx * dx + dy * dy < a.route_thr2 && a.route_end[g.route_off + wid] > wid + 1u) {
           wid += 1u;
           rw += 1u;
         }
@@ -927,8 +932,8 @@ __device__ __forceinline__ void integrate_and_store(const StepArgs& a, uint32_t 
         } else {
           wp += 1;
           // HighLevelPlanner::set_target(.., waypoints[next_waypoint], ..) (lib.rs:326-333): the route follower
-          // starts over at the head of its route (rmf/mod.rs:217-237 inserts (route, 0))
-          if (g.hl_kind == HL_ROUTE) rwp = 1u;
+          // starts over at the head of the leg to that waypoint (rmf/mod.rs:217-237 inserts (route, 0))
+          if (g.hl_kind == HL_ROUTE) rwp = a.ss_rwp[ss.wp_off + wp];
         }
       }
     }
@@ -1394,6 +1399,26 @@ __global__ void route_set_target_kernel(uint32_t m, const uint64_t* __restrict__
   wp[sl] = (wp[sl] & WP_MASK) | (1u << WP_ROUTE_SHIFT);
 }
 
+// The same for a route-table planner: agent k enters the cache at entry[k] (the head of the leg its target selects).
+// Every id must be live and in a group of the planner (of_planner[group] != 0); write = 0 only counts the bad ids, so
+// that a refused call changes nothing.
+__global__ void route_table_set_target_kernel(uint32_t m, const uint64_t* __restrict__ ids,
+                                              const uint32_t* __restrict__ entry,
+                                              const uint32_t* __restrict__ slot_of_id, uint64_t table_len,
+                                              const uint32_t* __restrict__ grp, const uint32_t* __restrict__ of_planner,
+                                              uint32_t n_groups, uint32_t write, uint32_t* __restrict__ wp,
+                                              unsigned int* bad) {
+  uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= m) return;
+  uint64_t v = ids[k];
+  uint32_t sl = v < table_len ? slot_of_id[v] : 0xffffffffu;
+  if (sl == 0xffffffffu || grp[sl] >= n_groups || !of_planner[grp[sl]]) {
+    atomicAdd(bad, 1u);
+    return;
+  }
+  if (write) wp[sl] = (wp[sl] & WP_MASK) | (entry[k] << WP_ROUTE_SHIFT);
+}
+
 __global__ void fill_u32_kernel(uint64_t n, uint32_t* p, uint32_t v) {
   uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) p[i] = v;
@@ -1559,7 +1584,7 @@ __global__ void ss_bits_sum_kernel(uint32_t n_words, uint32_t world, const uint3
 // generator asks for >= 1 (the reference's loop over spawn_number is commented out, lib.rs:207-219).
 // Ids are allocated sequentially (lib.rs:128-129) in that order.  gbits != nullptr (strips): the global spawn set
 // (ss_flags_kernel, summed over the ranks) decides and numbers the spawns; this rank materialises its own sources'.
-__global__ void ss_spawn_kernel(GridDev g, const SourceSinkDev* __restrict__ ss, const GroupDev* __restrict__ groups,
+__global__ void ss_spawn_kernel(GridDev g, const SourceSinkDev* __restrict__ ss, const uint32_t* __restrict__ ss_rwp,
                                 uint32_t n_ss, double dt, const uint32_t* __restrict__ gbits,
                                 uint32_t* __restrict__ blocked, AgentArrays cur, uint32_t* __restrict__ keep,
                                 uint32_t cap, uint32_t* cnt, unsigned long long* next_id, unsigned long long* ev_id, double* ev_xy, uint32_t ev_cap,
@@ -1600,8 +1625,8 @@ __global__ void ss_spawn_kernel(GridDev g, const SourceSinkDev* __restrict__ ss,
         cur.id[slot] = id;
         cur.grp[slot] = s.grp;
         // set_target(agent, waypoints[0], ..) right after the spawn (lib.rs:242-249): a route follower starts at
-        // the head of its route
-        cur.wp[slot] = groups[s.grp].hl_kind == HL_ROUTE ? (1u << WP_ROUTE_SHIFT) : 0u;
+        // the head of the leg to waypoint 0
+        cur.wp[slot] = ss_rwp[s.wp_off] << WP_ROUTE_SHIFT;
         keep[slot] = 1u;
         if (cur.pv)
           cur.pv[slot] = make_double2(__longlong_as_double(0x7ff8000000000000LL),

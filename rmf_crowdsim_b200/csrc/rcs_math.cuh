@@ -13,7 +13,8 @@ namespace rcs {
 #define RCS_INF (__longlong_as_double(0x7ff0000000000000LL))
 
 enum : uint32_t { LP_NONE = 0, LP_ZANLUNGO = 1 };
-enum : uint32_t { HL_NONE = 0, HL_CONSTANT = 1, HL_PARITY = 2, HL_HOST = 3, HL_ROUTE = 4 };
+// HL_ROUTE_TABLE is a host-side kind only: its groups run as HL_ROUTE (a route planner is a table of one leg).
+enum : uint32_t { HL_NONE = 0, HL_CONSTANT = 1, HL_PARITY = 2, HL_HOST = 3, HL_ROUTE = 4, HL_ROUTE_TABLE = 5 };
 
 // LocationHash2D geometry (location_hash_2d.rs:14-23, 33-51) in device form.
 struct GridDev {
@@ -53,7 +54,7 @@ struct GroupDev {
   uint32_t hl_kind;
   uint32_t w0_fast;      // 1: a weight-0 pair can only contribute +-0 or NaN (see pair_force_w0_is_zero)
   int32_t source_sink;   // index into the source-sink table, -1 if none
-  uint32_t route_off, route_n;  // HL_ROUTE: polyline in the route table (points, not doubles)
+  uint32_t route_off, route_n;  // HL_ROUTE: the planner's table in the route array (points, not doubles)
 };
 
 // Rust `f64 as usize` (saturating, NaN -> 0), location_hash_2d.rs:56-57.

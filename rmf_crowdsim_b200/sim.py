@@ -13,7 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, Mapping, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -148,6 +148,20 @@ class RouteFollowPlan(HighLevelPlanner):
 
     def __init__(self, route: Sequence[Vec2f]):
         self.route = [(float(p[0]), float(p[1])) for p in route]
+
+
+class RouteTablePlan(HighLevelPlanner):
+    """rmf::RMFPlanner (rmf/mod.rs:86-241) with a route cache the caller has filled, evaluated on the device.
+    `routes` maps each target point to the route (leg) that set_target(agent, target, ..) selects.  set_target makes the
+    leg whose target equals the point (IEEE == on both coordinates) the agent's current leg, at its route point 0;
+    get_desired_velocity is RouteFollowPlan's follower on that leg.  A SourceSink calls set_target with waypoints[0] at
+    the spawn and with waypoints[k + 1] at every advance (not at a loop_forever wrap), so a SourceSink with this planner
+    may have any number of waypoints, each of which must have a leg.  Route planning itself (`mapf`) stays outside."""
+
+    device_kind = "route_table"
+
+    def __init__(self, routes: Mapping[Vec2f, Sequence[Vec2f]]):
+        self.routes = {(float(t[0]), float(t[1])): [(float(p[0]), float(p[1])) for p in r] for t, r in routes.items()}
 
 
 class NoHighLevelPlan(HighLevelPlanner):
@@ -340,6 +354,13 @@ class Simulation:
         elif kind == "route":
             r = _f64(hl.route).reshape(-1)
             N.check(self._h, self._lib.rcs_hl_route(self._h, len(r) // 2, _p(r, N.c_f64p), C.byref(out)))
+        elif kind == "route_table":
+            legs = list(hl.routes.items())
+            targets = _f64([t for t, _ in legs]).reshape(-1)
+            counts = _u64([len(r) for _, r in legs])
+            xy = _f64([p for _, r in legs for p in r]).reshape(-1)
+            N.check(self._h, self._lib.rcs_hl_route_table(self._h, len(legs), _p(targets, N.c_f64p),
+                                                          _p(counts, N.c_u64p), _p(xy, N.c_f64p), C.byref(out)))
         else:
             if self._host_hl_handle is None:
                 N.check(self._h, self._lib.rcs_hl_host(self._h, C.byref(out)))
@@ -578,6 +599,17 @@ class Simulation:
         """HighLevelPlanner::set_target for agents of a RouteFollowPlan: enter the cache at route point 0."""
         ids = _u64(ids)
         N.check(self._h, self._lib.rcs_hl_route_set_target(self._h, len(ids), _p(ids, N.c_u64p)))
+
+    def route_table_set_target(self, planner: RouteTablePlan, ids, targets) -> None:
+        """HighLevelPlanner::set_target(agent, targets[i], ..) of a RouteTablePlan for the agents ids[i], which it must
+        drive: each enters the cache at the head of the leg its target selects.  An unknown id, an agent of another
+        planner or a target without a leg raises CrowdsimError and changes nothing."""
+        ids = _u64(ids)
+        xy = _f64(targets).reshape(-1)
+        if len(xy) != 2 * len(ids):
+            raise CrowdsimError(N.RCS_ERR_ARG, "route_table_set_target: one target point per id")
+        N.check(self._h, self._lib.rcs_hl_route_table_set_target(self._h, self._hl(planner), len(ids),
+                                                                 _p(ids, N.c_u64p), _p(xy, N.c_f64p)))
 
     def set_preferred_velocity(self, ids, vxy) -> None:
         vxy = _f64(vxy).reshape(-1)
