@@ -118,7 +118,7 @@ extern "C" {
     pub fn rcs_query_knn(sim: *mut rcs_sim, nq: u64, qxy: *const f64, k: u64, out_ids: *mut u64,
                          out_counts: *mut u64) -> c_int;
 
-    /// options: 1 = step kernel form, 2 = bin ahead, 3 = CUDA graphs for steady-state steps (include/rcs.h)
+    /// options: 1 = step kernel form, 3 = CUDA graphs for steady-state steps (include/rcs.h)
     pub fn rcs_set_option(sim: *mut rcs_sim, option: u32, value: u64) -> c_int;
     pub fn rcs_graph_stats(sim: *mut rcs_sim, out_graph_launches: *mut u64, out_captures: *mut u64) -> c_int;
 

@@ -257,19 +257,10 @@ int rcs_read_trace(rcs_sim* sim, uint64_t* ids, double* t_i, double* fx, double*
 
 /* ---- options ------------------------------------------------------------------------------------ */
 #define RCS_OPT_STEP_KERNEL 1u /* 0 = default (3), 1 = thread-per-agent, 2 = warp-cooperative through L1, 3 = stencil staged in shared memory */
-/* 1 = the step kernel's epilogue files every agent under the cell of the position the next step starts from (cell id +
- * histogram atomics), so that step's index rebuild starts at the prefix sum.  Off by default: measured slower -- the
- * atomics cost more inside the latency-bound step kernel than in the bandwidth-bound binning pass they replace. */
-#define RCS_OPT_BIN_AHEAD 2u
+/* Option numbers 2 and 4 are retired and are not reused: rcs_set_option refuses them as unknown options. */
 /* 1 (default) = a step whose launch sequence repeats (nothing to upload, no trace, no kernel timing) is captured into a
  * CUDA graph the second time it comes up and is one graph launch from then on; 0 = always launch kernel by kernel. */
 #define RCS_OPT_GRAPHS 3u
-/* 1 = the kernels of a step are launched as programmatic dependents of one another
- * (cudaLaunchAttributeProgrammaticStreamSerialization; every one of them starts with griddepcontrol.wait): the blocks of
- * the next kernel are dispatched while the current one drains, so the launch latencies of the dozen kernels of a step
- * overlap.  Same results.  Off by default: inside the captured graphs it was measured to change nothing at 2^24 agents and
- * +-2 % either way on small crowds (profiles/r02_step_tile_kernel.md); RCS_PDL=1 in the environment turns the default on. */
-#define RCS_OPT_PDL 4u
 int rcs_set_option(rcs_sim* sim, uint32_t option, uint64_t value);
 
 /* ---- measurement helpers ---------------------------------------------------------------------- */

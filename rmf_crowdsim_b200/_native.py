@@ -33,9 +33,7 @@ RCS_STEP_DEFAULT = 0
 RCS_STEP_NO_COMMIT = 1
 RCS_NUM_EVENTS = 64
 RCS_OPT_STEP_KERNEL = 1
-RCS_OPT_BIN_AHEAD = 2
 RCS_OPT_GRAPHS = 3
-RCS_OPT_PDL = 4
 
 
 class SimDesc(C.Structure):

@@ -107,10 +107,10 @@ struct StepKey {
   const void* cur_pos = nullptr;
   uint32_t flags = 0, n_ub = 0, n = 0;
   uint32_t n_ub_spawn = 0;  // the launch bound after this step's spawns: phase B's grids (spawn_launch_bound)
-  bool cur_has_dead = false, binned_ahead = false;
+  bool cur_has_dead = false;
   bool operator==(const StepKey& o) const {
     return epoch == o.epoch && dt_bits == o.dt_bits && cur_pos == o.cur_pos && flags == o.flags && n_ub == o.n_ub &&
-           n == o.n && n_ub_spawn == o.n_ub_spawn && cur_has_dead == o.cur_has_dead && binned_ahead == o.binned_ahead;
+           n == o.n && n_ub_spawn == o.n_ub_spawn && cur_has_dead == o.cur_has_dead;
   }
 };
 struct StepGraph {
@@ -183,8 +183,6 @@ struct rcs_sim {
   unsigned long long* d_next_id = nullptr;  // device copy of last_alloc_agent_id (source sinks allocate ids)
   uint64_t max_id_plus1 = 0;
   bool index_valid = false;  // srt + cell_start describe the current positions
-  // the last step's epilogue has binned `cur` for the next one: cellid[] and the histogram cell_count[] are current
-  bool binned_ahead = false;
   // id-addressed access
   uint32_t *slot_of_id = nullptr, *id_rank = nullptr, *order_by_id = nullptr, *presence = nullptr;
   uint64_t slot_table_cap = 0;
@@ -262,10 +260,8 @@ struct rcs_sim {
   cudaEvent_t events[RCS_NUM_EVENTS]{};
   uint32_t opt_step_kernel = 0;
   bool tile_attr_set = false;
-  uint32_t opt_bin_ahead = 0;  // RCS_OPT_BIN_AHEAD
   // CUDA graphs of steady-state steps
   uint32_t opt_graphs = 1;     // RCS_OPT_GRAPHS
-  uint32_t opt_pdl = 0;        // RCS_OPT_PDL
   uint64_t graph_epoch = 0;    // bumped by everything that can change a step's launch sequence or kernel arguments
   std::vector<rcs_host::StepGraph> step_graphs;
   rcs_host::StepKey recent_keys[2];  // keys of the last steps that ran eagerly (a key seen again is captured)

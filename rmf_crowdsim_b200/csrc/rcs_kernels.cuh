@@ -33,7 +33,7 @@ struct DevStatus {
 };
 
 // device-side agent counts (the host only knows upper bounds while steps with churn are in flight)
-enum : int { CNT_CUR = 0, CNT_TOT = 1, CNT_SAVE = 2, CNT_EV_SPAWN = 3, CNT_EV_DESTROY = 4, CNT_EV_SPAWN_SAVE = 5,
+enum : int { CNT_CUR = 0, CNT_TOT = 1, CNT_EV_SPAWN = 3, CNT_EV_DESTROY = 4, CNT_EV_SPAWN_SAVE = 5,
              CNT_EV_DESTROY_SAVE = 6, CNT_N = 8 };
 
 // one source sink on the device (source_sink.rs:36-60 + the per-step logic of lib.rs:199-254, 305-336)
@@ -78,17 +78,6 @@ struct AgentArrays {
   double2* pv;  // host-planner preferred velocities; NaN in .x = None.  nullptr if no host planner exists
 };
 
-// Programmatic dependent launch (RCS_OPT_PDL): the kernels of a step are launched with
-// cudaLaunchAttributeProgrammaticStreamSerialization, so the blocks of kernel k + 1 are dispatched while kernel k is
-// still running and sit in griddepcontrol.wait until k has completed and its stores are visible -- the launch latency
-// between the dozen small kernels of a step overlaps instead of adding up.  pdl_enter() is the FIRST statement of every
-// kernel launched that way, executed by every thread (a block that left without it would let its grid complete, and the
-// next grid start, before the previous one is done).  Without the launch attribute both instructions do nothing.
-__device__ __forceinline__ void pdl_enter() {
-  asm volatile("griddepcontrol.launch_dependents;");
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
-
 // Halo packing fused into the binning pass over the owned agents of a strip: an agent whose insert cell lies in
 // the outermost `width` columns is appended to the send buffer of that side (both, on a very narrow strip).
 struct PackArgs {
@@ -102,42 +91,10 @@ struct PackArgs {
 };
 
 // Strips: agent i of the owned agents sits in cell `idx`; if that is one of the outermost `width` columns of the
-// strip it is appended to the send buffer of that side (both, on a very narrow strip).
-__device__ __forceinline__ void halo_pack_one(const PackArgs& pk, uint32_t i, uint32_t idx, DevStatus* status) {
-  const uint32_t cx = idx / pk.nx;
-  const unsigned act = __activemask();  // the lanes that reached this call together
-  const unsigned lane = threadIdx.x & 31u;
-  const uint32_t par = pk.xseq ? (*pk.xseq & 1u) : 0u;
-#pragma unroll
-  for (int side = 0; side < 2; ++side) {
-    const bool send = side == 0 ? (pk.has_left && cx < pk.st.c0 + pk.width) : (pk.has_right && cx + pk.width >= pk.st.c1);
-    // One append per warp, not per agent: the boundary columns are contiguous in storage, so whole warps pack, and
-    // 50 000 atomics on one counter were a third of the binning pass (27 us per rank on 8 strips).
-    const unsigned m = __ballot_sync(act, send);
-    if (!m) continue;
-    const HaloBuf& b = side == 0 ? pk.left : pk.right;
-    const int leader = __ffs(m) - 1;
-    uint32_t base = 0;
-    if ((int)lane == leader) base = atomicAdd(b.count, (unsigned)__popc(m));
-    base = __shfl_sync(act, base, leader);
-    if (!send) continue;
-    uint32_t k = base + __popc(m & ((1u << lane) - 1u));
-    if (k >= b.cap) {
-      atomicAdd(&status->capacity_err, 1u);
-      continue;
-    }
-    k += par * b.cap;  // peer-store transport: the rows go straight into the neighbour's receive buffer
-    b.pos[k] = pk.cur.pos[i];
-    b.vel[k] = pk.cur.vel[i];
-    b.id[k] = pk.cur.id[i];
-    b.meta[k] = (unsigned long long)pk.cur.grp[i] | ((unsigned long long)pk.cur.wp[i] << 32);
-    if (pk.cur.pv) b.pv[k] = pk.cur.pv[i];
-  }
-}
-
-// The same for a whole block of the binning pass (every thread of the block calls it, `mine` = this thread has an agent
-// to test): ONE append per block and side.  The boundary columns are contiguous in storage, so ~100 blocks per side
-// pack; with one atomic per warp the 770 same-address atomics per side were most of the pass's extra time on 8 strips.
+// strip it is appended to the send buffer of that side (both, on a very narrow strip).  Every thread of a block of the
+// binning pass calls this (`mine` = this thread has an agent to test): ONE append per block and side.  The boundary
+// columns are contiguous in storage, so ~100 blocks per side pack; with one atomic per warp the 770 same-address
+// atomics per side were most of the pass's extra time on 8 strips.
 template <int THREADS>
 __device__ __forceinline__ void halo_pack_block(const PackArgs& pk, bool mine, uint32_t i, uint32_t idx,
                                                 DevStatus* status) {
@@ -181,17 +138,6 @@ __device__ __forceinline__ void halo_pack_block(const PackArgs& pk, bool mine, u
   }
 }
 
-// Strips, when the previous step's epilogue has already binned the owned agents (cellid, histogram): only the halo
-// pack of the binning pass is left to do.
-__global__ void halo_pack_kernel(uint32_t n_ub, const uint32_t* __restrict__ last, const uint32_t* __restrict__ cellid,
-                                 PackArgs pk, DevStatus* status) {
-  if (status->failed) return;
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n_ub || i >= *last) return;
-  const uint32_t c = cellid[i];
-  if (c != 0xffffffffu) halo_pack_one(pk, i, c, status);
-}
-
 constexpr int SCAN_THREADS = 256;
 constexpr int SCAN_ITEMS = 16;
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
@@ -227,19 +173,18 @@ __device__ __forceinline__ bool bin_one(const GridDev& g, uint32_t i, double2 p,
   return true;
 }
 
-// Agents [*first (0 if null), min(n_ub, *last)) of the unsorted arrays.  Entries whose keep flag is 0 (despawned
-// at a sink, migrated to another strip, ghosts of the previous step) are dropped here: the counting sort of the
-// next step is the stream compaction.
+// Agents [0, min(n_ub, *last)) of the unsorted arrays.  Entries whose keep flag is 0 (despawned at a sink, migrated
+// to another strip, ghosts of the previous step) are dropped here: the counting sort of the next step is the stream
+// compaction.
 // PACK: the strip form (every thread of a block reaches the block-wide halo append); the plain form leaves early and
 // keeps the registers for 2048 resident threads (the pass is latency-bound on its loads and atomics).
 template <bool PACK>
 __global__ void __launch_bounds__(BIN_THREADS, 8) bin_count_kernel(
-    GridDev g, uint32_t n_ub, const uint32_t* __restrict__ first, const uint32_t* __restrict__ last,
-    const double2* __restrict__ pos, const uint32_t* __restrict__ keep, uint32_t* __restrict__ cellid,
-    uint32_t* __restrict__ cell_count, uint64_t cell_lo, uint64_t cell_hi, PackArgs pk, DevStatus* status) {
-  pdl_enter();
+    GridDev g, uint32_t n_ub, const uint32_t* __restrict__ last, const double2* __restrict__ pos,
+    const uint32_t* __restrict__ keep, uint32_t* __restrict__ cellid, uint32_t* __restrict__ cell_count,
+    uint64_t cell_lo, uint64_t cell_hi, PackArgs pk, DevStatus* status) {
   if (status->failed) return;
-  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x + (first ? *first : 0u);
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   bool live = i < n_ub && i < *last;
   if (!PACK && !live) return;
   if (live && keep && !keep[i]) {
@@ -288,7 +233,6 @@ __device__ __forceinline__ uint32_t block_exclusive_scan(uint32_t v, uint32_t& t
 }
 
 __global__ void scan_reduce_kernel(const uint32_t* __restrict__ in, uint64_t len, uint32_t* __restrict__ tile_sums) {
-  pdl_enter();
   uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)threadIdx.x * SCAN_ITEMS;
   uint32_t s = 0;
   if (base + SCAN_ITEMS <= len) {
@@ -330,7 +274,6 @@ template <bool RAW_SUMS>
 __global__ void scan_apply_kernel(const uint32_t* __restrict__ in, uint64_t len,
                                   const uint32_t* __restrict__ tile_sums, uint32_t* __restrict__ cell_start,
                                   uint32_t* __restrict__ cursor) {
-  pdl_enter();
   uint64_t base = (uint64_t)blockIdx.x * SCAN_TILE + (uint64_t)threadIdx.x * SCAN_ITEMS;
   uint32_t v[SCAN_ITEMS];
   uint32_t s = 0;
@@ -393,7 +336,6 @@ __global__ void scan_apply_kernel(const uint32_t* __restrict__ in, uint64_t len,
 __global__ void scatter_perm_kernel(uint32_t n_ub, const uint32_t* __restrict__ n_ptr,
                                     const uint32_t* __restrict__ cellid, uint32_t* __restrict__ cursor,
                                     uint32_t* __restrict__ perm, const DevStatus* status) {
-  pdl_enter();
   if (status->failed) return;
   uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_ub || i >= *n_ptr) return;
@@ -409,7 +351,6 @@ __global__ void scatter_perm_kernel(uint32_t n_ub, const uint32_t* __restrict__ 
 __global__ void sort_cells_by_id_kernel(uint64_t cell_lo, uint64_t cell_hi, const uint32_t* __restrict__ cell_start,
                                         const uint64_t* __restrict__ id, uint32_t* __restrict__ perm,
                                         uint32_t* __restrict__ big_list, uint32_t big_cap, DevStatus* status) {
-  pdl_enter();
   if (status->failed) return;
   uint64_t c = cell_lo + (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= cell_hi) return;
@@ -519,7 +460,6 @@ __global__ void __launch_bounds__(1024) sort_big_cells_kernel(uint64_t cell_lo, 
                                                               uint32_t* __restrict__ ranks,
                                                               const uint32_t* __restrict__ big_list, uint32_t big_cap,
                                                               DevStatus* status) {
-  pdl_enter();
   __shared__ unsigned long long skeys[BIG_SMEM_KEYS];
   __shared__ uint32_t partial[32][HUGE_ELEMS];
   __shared__ bool last_block;
@@ -618,7 +558,6 @@ __global__ void __launch_bounds__(GATHER_THREADS) gather_sorted_kernel(
     uint32_t* __restrict__ srt_cell, const uint32_t* __restrict__ n_sorted, GridDev g,
     const uint32_t* __restrict__ cell_start, const GroupDev* __restrict__ groups, uint4* __restrict__ slices,
     TileRange* __restrict__ tile_ranges, const DevStatus* status) {
-  pdl_enter();
   __shared__ uint32_t red[GATHER_THREADS / 32][6];
   if (status->failed) return;  // block-uniform
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -682,11 +621,6 @@ struct StepArgs {
   uint32_t* wide_list;             // warp kernel: agents left to the chunked cooperative routine
   const uint4* slices;             // candidate slices prepared by gather_sorted_kernel (sorted path only)
   const TileRange* tile_ranges;    // per block of step_tile_kernel: rows to stage (gather_sorted_kernel)
-  // Binning ahead: the epilogue files every agent that stays under the cell of the position the NEXT step starts
-  // from (A1 / A2 of that step: cell id + histogram), so that step's rebuild starts at the prefix sum.
-  uint32_t* next_cellid;           // nullptr: off
-  uint32_t* next_count;
-  uint64_t cell_lo, cell_hi;       // cells this handle indexes
   const double* routes;            // HL_ROUTE polylines, interleaved x,y
   const uint32_t* route_end;       // per route point: one past the last point of its leg, within its planner's table
   double route_thr2;               // smallest double T with sqrt(T) >= 1e-1 (rmf/mod.rs:202)
@@ -729,7 +663,6 @@ __device__ __forceinline__ uint32_t agent_role(const StepArgs& a, uint32_t i) {
 // it is not part of the next state.
 __device__ __forceinline__ void drop_entry(const StepArgs& a, uint32_t i) {
   if (a.keep) a.keep[i] = 0u;
-  if (a.next_cellid) a.next_cellid[i] = CELL_DEAD;
 }
 
 struct Self {
@@ -964,19 +897,6 @@ __device__ __forceinline__ void integrate_and_store(const StepArgs& a, uint32_t 
   }
   if (a.no_commit) keep = own;  // the pre-step snapshot stays: this rank keeps exactly what it owned
   if (a.keep) a.keep[i] = keep ? 1u : 0u;
-  if (a.next_cellid) {
-    // location_to_index (A1) of the position the next step starts from: the new one, or -- without commit -- the old
-    uint64_t c = idx;
-    bool cin = inb;
-    if (a.no_commit) cin = location_to_index(a.grid, me.px, me.py, c);
-    if (keep && cin && c >= a.cell_lo && c < a.cell_hi) {
-      a.next_cellid[i] = (uint32_t)c;
-      atomicAdd(&a.next_count[c], 1u);
-    } else {
-      a.next_cellid[i] = CELL_DEAD;
-      if (keep && cin) atomicAdd(&a.status->halo_err, 1u);  // outside the cells this rank indexes (bin_count_kernel)
-    }
-  }
 }
 
 __device__ __forceinline__ void warp_stats(const StepArgs& a, uint32_t cand, uint32_t nbc, uint32_t finite) {
@@ -1436,7 +1356,6 @@ __global__ void fill_f64_kernel(uint64_t n, double* p, double v) {
 // failed" (so that a failure reaches the neighbours with the next exchange and the whole job stops within `world` steps)
 __global__ void begin_step_kernel(DevStatus* st, uint32_t* cnt, uint32_t* send_l_hdr, uint32_t* send_r_hdr,
                                   uint32_t* xseq) {
-  pdl_enter();
   if (xseq) *xseq += 1u;  // peer-store transport: one exchange round per step, failed steps included
   if (send_l_hdr) {
     send_l_hdr[0] = 0u;
@@ -1459,7 +1378,6 @@ __global__ void begin_step_kernel(DevStatus* st, uint32_t* cnt, uint32_t* send_l
   st->finite_tti = 0;
   st->neighbour_total = 0;
   st->candidate_total = 0;
-  cnt[CNT_SAVE] = cnt[CNT_CUR];
   cnt[CNT_TOT] = cnt[CNT_CUR];
   cnt[CNT_EV_SPAWN_SAVE] = cnt[CNT_EV_SPAWN];
   cnt[CNT_EV_DESTROY_SAVE] = cnt[CNT_EV_DESTROY];
@@ -1470,7 +1388,6 @@ __global__ void begin_step_kernel(DevStatus* st, uint32_t* cnt, uint32_t* send_l
 // cnt_cur != nullptr on steps with churn: the state now holds *n_sorted entries (some flagged keep = 0).
 __global__ void end_step_kernel(DevStatus* st, int oob_fails, unsigned long long* steps_done, uint32_t* cnt_cur,
                                 const uint32_t* n_sorted) {
-  pdl_enter();
   if (st->failed) return;
   if ((oob_fails && st->oob_count) || st->halo_err || st->capacity_err) {
     st->local_failed = 1;
@@ -1706,7 +1623,6 @@ __global__ void halo_unpack_kernel(AgentArrays cur, uint32_t* __restrict__ keep,
                                    uint32_t* __restrict__ cell_count, uint64_t cell_lo, uint64_t cell_hi,
                                    const uint32_t* __restrict__ send_l_hdr, const uint32_t* __restrict__ send_r_hdr,
                                    uint32_t* remote_l_hdr, uint32_t* remote_r_hdr) {
-  pdl_enter();
   uint32_t par = 0u;
   if (xseq) {
     if (blockIdx.x == 0 && threadIdx.x < 2)  // this rank's own round first: nobody waits for a rank that waits

@@ -174,7 +174,6 @@ __device__ __noinline__ void st_flush_hits(TileWarp& w, uint32_t n_hit, const do
 // STRIPS: the handle is a strip (ownership roles, keep flags by the new column); the plain form has none of that code.
 template <bool STRIPS>
 __global__ void __launch_bounds__(32 * ST_WARPS, RCS_TILE_BLOCKS) step_tile_kernel(StepArgs a) {
-  pdl_enter();
   extern __shared__ __align__(16) unsigned char st_smem_raw[];
   TileShared& sh = *reinterpret_cast<TileShared*>(st_smem_raw);
   const unsigned warp = threadIdx.x >> 5;

@@ -516,7 +516,6 @@ struct WideMasks {
 // the weight-0 proof): 32 per warp, cooperatively, chunked stencil columns.  a.slow_list: one per thread with the
 // sequential routine.  Grid-stride over the device-side counts.
 __global__ void __launch_bounds__(32 * SW_WARPS, 4) step_aside_kernel(StepArgs a) {
-  pdl_enter();
   __shared__ WarpShared sh[SW_WARPS];
   __shared__ WideMasks shm[SW_WARPS];
   WarpShared& w = sh[threadIdx.x >> 5];

@@ -46,6 +46,14 @@ def test_unknown_ids_are_errors_and_leave_the_state_alone():
     assert sim.agent_count() == 2
     sim.spatial_index.remove_agent(12345)  # SpatialIndex::remove_agent of an unknown id is a no-op (:260-267)
     assert sim.agent_count() == 2
+    for option in (2, 4):  # retired option numbers are unknown options, whatever the value
+        for value in (0, 1):
+            with pytest.raises(R.CrowdsimError) as e:
+                sim.set_option(option, value)
+            assert e.value.code == N.RCS_ERR_ARG and str(e.value) == "unknown option or value"
+    steps = sim.stats().steps
+    sim.step(R.Duration(1, 0))
+    assert sim.stats().steps == steps + 1 and sim.agent_count() == 2
 
 
 def test_empty_and_ragged_batches():

@@ -426,42 +426,3 @@ def test_streaming_kernel_of_no_local_plan_crowds_matches_the_generic_kernel_and
         assert np.array_equal(sa[k].view(np.uint64), so[k].view(np.uint64)), k
     assert a.launch_count() < b.launch_count() + 100  # both ran; no index was built on either path
 
-
-def test_bin_ahead_option_is_bit_identical():
-    """RCS_OPT_BIN_AHEAD (the step kernel's epilogue bins the agents for the next step's index rebuild) changes how the
-    rebuild is scheduled, not what it computes: committed steps, frozen steps and a state injection in between give
-    the same bits with the option on and off."""
-    from rmf_crowdsim_b200 import _native as N
-
-    scene = SC.uniform_crowd(128, "lane", margin=16.0, seed=3)
-    sims = []
-    for on in (0, 1):
-        g = SC.build_simulation(scene)
-        g.set_option(N.RCS_OPT_BIN_AHEAD, on)
-        sims.append(g)
-    dt = R.Duration(0, 100_000_000)
-
-    def same():
-        sa, sb = sims[0].read_state(order=N.RCS_ORDER_STORAGE), sims[1].read_state(order=N.RCS_ORDER_STORAGE)
-        for k in ("id", "x", "y", "vx", "vy"):
-            assert np.array_equal(sa[k].view(np.uint64), sb[k].view(np.uint64)), k
-        assert sims[0].stats().neighbour_total == sims[1].stats().neighbour_total
-
-    for g in sims:
-        for _ in range(6):
-            g.step_async(dt)
-        g.sync()
-    same()
-    for g in sims:
-        for _ in range(3):
-            g.step_async(dt, no_commit=True)
-        g.step_async(dt)
-        g.sync()
-    same()
-    st = sims[0].read_state()
-    for g in sims:
-        g.set_state(None, st["x"] + 0.25, st["y"], st["vx"], st["vy"])
-        for _ in range(4):
-            g.step_async(dt)
-        g.sync()
-    same()
