@@ -65,6 +65,21 @@ pub struct rcs_source_sink_desc {
     pub agent_eyesight_range: f64,
 }
 
+pub const RCS_CROWD_MONOTONIC: u32 = 0;
+pub const RCS_CROWD_POISSON: u32 = 1;
+pub const RCS_CROWD_HOST: u32 = 2;
+
+/// `CrowdGenerator` of a source sink (source_sink.rs:63-100): `MonotonicCrowd::new(rate)`, `PoissonCrowd::new(rate)` with
+/// a keyed draw (`seed`; reproducible), or a user generator evaluated by the caller (`rcs_set_spawn_counts`).
+#[repr(C)]
+#[derive(Default, Debug, Clone, Copy)]
+pub struct rcs_crowd_generator {
+    pub kind: u32,
+    pub reserved: u32,
+    pub rate: f64,
+    pub seed: u64,
+}
+
 extern "C" {
     pub fn rcs_abi_version() -> u32;
     pub fn rcs_sim_create(desc: *const rcs_sim_desc, out: *mut *mut rcs_sim) -> c_int;
@@ -109,6 +124,9 @@ extern "C" {
                            n_destroyed: *mut u64) -> c_int;
     pub fn rcs_add_source_sink(sim: *mut rcs_sim, desc: *const rcs_source_sink_desc, out_id: *mut u64) -> c_int;
     pub fn rcs_remove_source_sink(sim: *mut rcs_sim, id: u64) -> c_int;
+    pub fn rcs_add_source_sink_gen(sim: *mut rcs_sim, desc: *const rcs_source_sink_desc, gen: *const rcs_crowd_generator,
+                                   out_id: *mut u64) -> c_int;
+    pub fn rcs_set_spawn_counts(sim: *mut rcs_sim, n: u64, ids: *const u64, counts: *const u64) -> c_int;
 
     pub fn rcs_cell_of(sim: *mut rcs_sim, n: u64, xy: *const f64, out_idx: *mut i64) -> c_int;
     pub fn rcs_index_add_or_update(sim: *mut rcs_sim, n: u64, ids: *const u64, xy: *const f64) -> c_int;

@@ -67,7 +67,26 @@ pub enum HighLevelPlan {
     Host(Arc<Mutex<dyn HighLevelPlanner>>),
 }
 
-/// source_sink/source_sink.rs:36-60 with `MonotonicCrowd::new(rate)`
+/// source_sink/source_sink.rs:63-66, verbatim: a user-implemented generator (`CrowdGen::Host`) is called once per step
+/// for every alive source sink that has it, in ascending source-sink id, before the step.  Only "at least one" matters:
+/// a source spawns at most one agent per step (lib.rs:207-219).
+pub trait CrowdGenerator {
+    fn get_number_to_spawn(&mut self, time_elapsed: Duration) -> usize;
+}
+
+/// The generator of a source sink (`Simulation::add_source_sink_gen`).
+#[derive(Clone)]
+pub enum CrowdGen {
+    /// `MonotonicCrowd::new(rate)` (source_sink.rs:85-100), on the device
+    Monotonic(f64),
+    /// `PoissonCrowd::new(rate)` (source_sink.rs:63-82) as a keyed draw on the device: reproducible for a given `seed`
+    /// (include/rcs.h); `rate` finite and > 0, and a step with `dt * rate <= 0` is refused
+    Poisson { rate: f64, seed: u64 },
+    /// any user generator, evaluated on the host every step
+    Host(Arc<Mutex<dyn CrowdGenerator>>),
+}
+
+/// source_sink/source_sink.rs:36-60 with `MonotonicCrowd::new(rate)` (`add_source_sink_gen` names the generator)
 pub struct SourceSink {
     pub source: Vec2f,
     pub radius_sink: f64,
@@ -85,6 +104,7 @@ pub struct Simulation {
     hl_host_handle: Option<u32>,
     eyesight: HashMap<AgentId, f64>,
     listeners: Vec<Arc<Mutex<dyn EventListener>>>,
+    host_gen: std::collections::BTreeMap<u64, Arc<Mutex<dyn CrowdGenerator>>>,
 }
 
 fn check(h: *mut sys::rcs_sim, rc: i32) -> Result<(), String> {
@@ -102,7 +122,8 @@ impl Simulation {
                                        capacity: capacity as u64, device, flags: 0 };
         let mut h: *mut sys::rcs_sim = ptr::null_mut();
         check(ptr::null_mut(), unsafe { sys::rcs_sim_create(&desc, &mut h) })?;
-        Ok(Simulation { h, host_hl: HashMap::new(), hl_host_handle: None, eyesight: HashMap::new(), listeners: vec![] })
+        Ok(Simulation { h, host_hl: HashMap::new(), hl_host_handle: None, eyesight: HashMap::new(), listeners: vec![],
+                       host_gen: std::collections::BTreeMap::new() })
     }
 
     fn lp(&mut self, lp: LocalPlan) -> Result<u32, String> {
@@ -169,7 +190,7 @@ impl Simulation {
         Ok(ids)
     }
 
-    /// lib.rs:159-162 (MonotonicCrowd generators run on the device; PoissonCrowd uses thread_rng and has no device form)
+    /// lib.rs:159-162 with `MonotonicCrowd::new(ss.monotonic_rate)`; `add_source_sink_gen` takes any generator
     pub fn add_source_sink(&mut self, ss: &SourceSink) -> Result<usize, String> {
         let (hl, lp) = (self.hl(&ss.high_level_planner)?, self.lp(ss.local_planner)?);
         let wp: Vec<f64> = ss.waypoints.iter().flat_map(|p| [p.x, p.y]).collect();
@@ -181,9 +202,32 @@ impl Simulation {
         Ok(id as usize)
     }
 
+    /// lib.rs:159-162 with the generator named (`ss.monotonic_rate` is ignored): Monotonic and Poisson run on the device,
+    /// a `CrowdGen::Host` generator is called by `step`
+    pub fn add_source_sink_gen(&mut self, ss: &SourceSink, generator: CrowdGen) -> Result<usize, String> {
+        let (hl, lp) = (self.hl(&ss.high_level_planner)?, self.lp(ss.local_planner)?);
+        let wp: Vec<f64> = ss.waypoints.iter().flat_map(|p| [p.x, p.y]).collect();
+        let desc = sys::rcs_source_sink_desc { source_x: ss.source.x, source_y: ss.source.y, radius_sink: ss.radius_sink,
+            monotonic_rate: 0.0, hl, lp, n_waypoints: ss.waypoints.len() as u64, waypoints_xy: wp.as_ptr(),
+            loop_forever: ss.loop_forever as i32, agent_eyesight_range: ss.agent_eyesight_range };
+        let gen = match &generator {
+            CrowdGen::Monotonic(rate) => sys::rcs_crowd_generator { kind: sys::RCS_CROWD_MONOTONIC, reserved: 0, rate: *rate, seed: 0 },
+            CrowdGen::Poisson { rate, seed } => sys::rcs_crowd_generator { kind: sys::RCS_CROWD_POISSON, reserved: 0, rate: *rate, seed: *seed },
+            CrowdGen::Host(_) => sys::rcs_crowd_generator { kind: sys::RCS_CROWD_HOST, reserved: 0, rate: 0.0, seed: 0 },
+        };
+        let mut id = 0u64;
+        check(self.h, unsafe { sys::rcs_add_source_sink_gen(self.h, &desc, &gen, &mut id) })?;
+        if let CrowdGen::Host(g) = generator {
+            self.host_gen.insert(id, g);
+        }
+        Ok(id as usize)
+    }
+
     /// lib.rs:164-168
     pub fn remove_source_sink(&mut self, id: &usize) -> Result<(), String> {
-        check(self.h, unsafe { sys::rcs_remove_source_sink(self.h, *id as u64) })
+        check(self.h, unsafe { sys::rcs_remove_source_sink(self.h, *id as u64) })?;
+        self.host_gen.remove(&(*id as u64));
+        Ok(())
     }
 
     /// lib.rs:170-173
@@ -241,6 +285,12 @@ impl Simulation {
                 }
             }
             check(self.h, unsafe { sys::rcs_set_preferred_velocity(self.h, ids.len() as u64, ids.as_ptr(), vxy.as_ptr()) })?;
+        }
+        if !self.host_gen.is_empty() {
+            // user CrowdGenerators: once per step, ascending source-sink id; the counts are for this step only
+            let ids: Vec<u64> = self.host_gen.keys().copied().collect();
+            let counts: Vec<u64> = self.host_gen.values().map(|g| g.lock().unwrap().get_number_to_spawn(dur) as u64).collect();
+            check(self.h, unsafe { sys::rcs_set_spawn_counts(self.h, ids.len() as u64, ids.as_ptr(), counts.as_ptr()) })?;
         }
         check(self.h, unsafe { sys::rcs_step(self.h, dur.as_secs(), dur.subsec_nanos()) })?;
         self.dispatch_events()

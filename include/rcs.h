@@ -224,6 +224,41 @@ typedef struct rcs_source_sink_desc {
 int rcs_add_source_sink(rcs_sim* sim, const rcs_source_sink_desc* desc, uint64_t* out_id);
 int rcs_remove_source_sink(rcs_sim* sim, uint64_t id);
 
+/* CrowdGenerator (source_sink.rs:63-100).  Only "get_number_to_spawn >= 1" matters: a source spawns at most one agent
+ * per step (the reference's loop over spawn_number is commented out, lib.rs:207-219).
+ *  MONOTONIC: MonotonicCrowd::new(rate), exactly as rcs_add_source_sink with monotonic_rate = rate.
+ *  POISSON  : PoissonCrowd::new(rate) with a keyed draw instead of thread_rng, so that runs are reproducible.  For
+ *             source sink id `sid` in the step that starts with rcs_stats.steps == k: w = word 0 of Philox4x64-10 of
+ *             counter (k + 1, sid, 0, 0) under key (seed, 0) (= numpy.random.Philox(key=[seed, 0],
+ *             counter=[k, sid, 0, 0]).random_raw()), u = w >> 11, lambda = dt * rate, T = ceil(exp(-lambda) * 2^53)
+ *             (the host C library's exp); the source wants to spawn iff u >= T, i.e. with probability 1 - exp(-lambda)
+ *             = P(Poisson(lambda) >= 1).  lambda < 2^-54: never; lambda > ~745: always.  A draw depends on (seed, k,
+ *             sid) only: adding or removing other source sinks, a retried failed step (it does not advance steps),
+ *             CUDA graph replay and the number of strips change nothing.  rate must be finite and > 0 (else
+ *             RCS_ERR_ARG, nothing added); a step (rcs_step, rcs_step_async, rcs_dist_step_local) of a handle with an
+ *             alive Poisson source and dt * rate <= 0 (dt = 0) is refused with RCS_ERR_ARG before anything runs, as
+ *             Poisson::new fails in the reference (source_sink.rs:79).
+ *  HOST     : a user-implemented generator evaluated by the caller, who uploads its counts with rcs_set_spawn_counts
+ *             before each step; rate and seed are ignored. */
+#define RCS_CROWD_MONOTONIC 0u
+#define RCS_CROWD_POISSON 1u
+#define RCS_CROWD_HOST 2u
+typedef struct rcs_crowd_generator {
+  uint32_t kind;     /* RCS_CROWD_* */
+  uint32_t reserved; /* 0 */
+  double rate;
+  uint64_t seed;
+} rcs_crowd_generator;
+/* rcs_add_source_sink with the generator named explicitly; desc->monotonic_rate is ignored.  Same rules otherwise
+ * (strips: the probe lies inside its owner's strip). */
+int rcs_add_source_sink_gen(rcs_sim* sim, const rcs_source_sink_desc* desc, const rcs_crowd_generator* gen,
+                            uint64_t* out_id);
+/* counts[i] = get_number_to_spawn of HOST-generator source sink ids[i], for the next step only: the step consumes the
+ * counts whether or not it stands, and a host source without a count spawns nothing.  An id listed twice takes its last
+ * count.  On strips every rank is given the counts; the rank that owns the source decides.  An unknown or removed id, a
+ * source whose generator is not HOST, or NULL arrays with n > 0 -> RCS_ERR_ARG and nothing is written. */
+int rcs_set_spawn_counts(rcs_sim* sim, uint64_t n, const uint64_t* ids, const uint64_t* counts);
+
 /* ---- SpatialIndex trait, batched (spatial_index.rs:4-14) ------------------------------------- */
 
 /* LocationHash2D::location_to_index for n points (location_hash_2d.rs:54-66): data index or -1. */

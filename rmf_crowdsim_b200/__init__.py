@@ -14,6 +14,7 @@ from .sim import (  # noqa: F401
     NoHighLevelPlan,
     NoLocalPlan,
     ParityVelocityPlan,
+    PoissonCrowd,
     RouteFollowPlan,
     RouteTablePlan,
     Simulation,
@@ -24,5 +25,5 @@ from .sim import (  # noqa: F401
 __all__ = [
     "Agent", "ConstantVelocityPlan", "CrowdGenerator", "CrowdsimError", "Duration", "EventListener",
     "HighLevelPlanner", "LocalPlanner", "LocationHash2D", "MonotonicCrowd", "NoHighLevelPlan", "NoLocalPlan",
-    "ParityVelocityPlan", "RouteFollowPlan", "RouteTablePlan", "Simulation", "SourceSink", "Zanlungo",
+    "ParityVelocityPlan", "PoissonCrowd", "RouteFollowPlan", "RouteTablePlan", "Simulation", "SourceSink", "Zanlungo",
 ]

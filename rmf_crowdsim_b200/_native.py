@@ -79,6 +79,20 @@ class SourceSinkDesc(C.Structure):
     ]
 
 
+RCS_CROWD_MONOTONIC = 0
+RCS_CROWD_POISSON = 1
+RCS_CROWD_HOST = 2
+
+
+class CrowdGeneratorDesc(C.Structure):
+    _fields_ = [
+        ("kind", C.c_uint32),
+        ("reserved", C.c_uint32),
+        ("rate", C.c_double),
+        ("seed", C.c_uint64),
+    ]
+
+
 # name -> (restype, argtypes); every symbol include/rcs.h declares
 SIGNATURES = {
     "rcs_abi_version": (C.c_uint32, []),
@@ -117,6 +131,8 @@ SIGNATURES = {
     ),
     "rcs_add_source_sink": (C.c_int, [C.c_void_p, C.POINTER(SourceSinkDesc), c_u64p]),
     "rcs_remove_source_sink": (C.c_int, [C.c_void_p, C.c_uint64]),
+    "rcs_add_source_sink_gen": (C.c_int, [C.c_void_p, C.POINTER(SourceSinkDesc), C.POINTER(CrowdGeneratorDesc), c_u64p]),
+    "rcs_set_spawn_counts": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p, c_u64p]),
     "rcs_cell_of": (C.c_int, [C.c_void_p, C.c_uint64, c_f64p, c_i64p]),
     "rcs_index_add_or_update": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p, c_f64p]),
     "rcs_index_remove": (C.c_int, [C.c_void_p, C.c_uint64, c_u64p]),

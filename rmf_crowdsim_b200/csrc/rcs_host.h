@@ -128,6 +128,25 @@ struct InLoopMem {
   uint64_t cap = 0, cells = 0;
 };
 
+// Small host-to-device uploads on the step stream through two pinned staging buffers used in turn: a buffer is
+// rewritten only after its previous copy has run, so an upload per step waits at most for the step before last.
+struct UploadRing {
+  void* buf[2] = {nullptr, nullptr};
+  cudaEvent_t ev[2] = {nullptr, nullptr};
+  bool used[2] = {false, false};
+  uint64_t cap = 0;  // bytes per buffer
+  uint32_t turn = 0;
+};
+
+inline void ring_free(UploadRing& r) {
+  for (int i = 0; i < 2; ++i) {
+    if (r.used[i]) cudaEventSynchronize(r.ev[i]);
+    if (r.buf[i]) cudaFreeHost(r.buf[i]);
+    if (r.ev[i]) cudaEventDestroy(r.ev[i]);
+  }
+  r = UploadRing{};
+}
+
 inline void inloop_free(InLoopMem*& m) {
   if (!m) return;
   cudaFree(m->np_a); cudaFree(m->np_b); cudaFree(m->nv); cudaFree(m->rank); cudaFree(m->cellid); cudaFree(m->perm);
@@ -213,6 +232,19 @@ struct rcs_sim {
   bool sources_dirty = false;
   uint32_t n_sources_alive = 0;
   bool ever_had_sources = false;
+  // CrowdGenerators other than MonotonicCrowd (ss_wants_spawn).  PoissonCrowd: per-source thresholds of the dt they
+  // were last computed for, uploaded through thr_ring when dt's bits change.  Host generators: the counts of the next
+  // step (1 = at least one), mirrored on the host until a step consumes them.
+  uint32_t n_poisson_alive = 0, n_host_gen_alive = 0;
+  unsigned long long* d_ss_thr = nullptr;
+  std::vector<unsigned long long> ss_thr;
+  uint64_t ss_thr_dt_bits = 0;
+  bool ss_thr_valid = false;
+  rcs_host::UploadRing thr_ring;
+  uint32_t* d_ss_count = nullptr;
+  std::vector<uint32_t> ss_count;
+  bool ss_count_consumed = false;  // a step ran since the last rcs_set_spawn_counts (the device copy is all zero)
+  rcs_host::UploadRing count_ring;
   // events (EventListener::agent_spawned / agent_destroyed)
   unsigned long long *ev_spawn_id = nullptr, *ev_destroyed = nullptr;
   double* ev_spawn_xy = nullptr;

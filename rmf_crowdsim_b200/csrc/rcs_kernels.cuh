@@ -47,7 +47,11 @@ struct SourceSinkDev {
   uint32_t loop_forever;
   uint32_t alive;           // 0 after remove_source_sink
   uint32_t owned;           // strips: this rank owns the source's cell column and spawns for it (1 on a single handle)
+  uint32_t gen;             // CrowdGenerator: GEN_* (= RCS_CROWD_*), see ss_wants_spawn
+  uint32_t pad_;
+  unsigned long long seed;  // PoissonCrowd: Philox key word 0
 };
+enum : uint32_t { GEN_MONOTONIC = 0, GEN_POISSON = 1, GEN_HOST = 2 };
 
 // spatial strips (SURVEY.md section 8e): this rank owns cell columns [c0, c1); h = halo ring width
 struct StripDev {
@@ -1473,18 +1477,57 @@ __global__ void ss_probe_kernel(GridDev g, SourceGridDev sg, const SourceSinkDev
   }
 }
 
+// What the generators other than MonotonicCrowd read in the spawn phase.  Both arrays are indexed by source id and are
+// nullptr while the handle has no source of that kind.
+struct SpawnGenDev {
+  const unsigned long long* thr;         // PoissonCrowd: ceil(exp(-dt * rate) * 2^53) for the step's dt (host, glibc exp)
+  uint32_t* host_cnt;                    // host generators: 1 = get_number_to_spawn returned >= 1 for this step
+  const unsigned long long* steps_done;  // steps executed on the handle (the same on every rank of a strip group)
+};
+
+// Word 0 of Philox4x64-10 (Salmon et al., SC'11) of counter (c0, c1, 0, 0) under key (k0, 0).
+__device__ __forceinline__ unsigned long long philox4x64_10_w0(unsigned long long c0, unsigned long long c1,
+                                                               unsigned long long k0) {
+  unsigned long long c2 = 0, c3 = 0, k1 = 0;
+  #pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const unsigned long long lo0 = 0xD2E7470EE14C6C93ull * c0, hi0 = __umul64hi(0xD2E7470EE14C6C93ull, c0);
+    const unsigned long long lo1 = 0xCA5A826395121157ull * c2, hi1 = __umul64hi(0xCA5A826395121157ull, c2);
+    c0 = hi1 ^ c1 ^ k0;
+    c1 = lo1;
+    c2 = hi0 ^ c3 ^ k1;
+    c3 = lo0;
+    k0 += 0x9E3779B97F4A7C15ull;
+    k1 += 0xBB67AE8584CAA73Bull;
+  }
+  return c0;
+}
+
+// Does source k's generator return >= 1 in this step?  Only that matters: the reference's loop over spawn_number is
+// commented out (lib.rs:207-219), a source spawns at most one agent per step.
+//  MonotonicCrowd: round(dt * rate) as usize > 0 (source_sink.rs:97-100).
+//  PoissonCrowd:   P(Poisson(dt * rate) >= 1) = 1 - exp(-dt * rate) as a keyed draw: u = (word 0 of Philox4x64-10,
+//                  counter (steps + 1, k, 0, 0), key (seed, 0)) >> 11 is uniform on [0, 2^53); the source wants to spawn
+//                  iff u >= thr[k].  Keyed, not stateful: the draw of (step, source) does not depend on other sources
+//                  or on how often a failed step was retried, and a replayed CUDA graph reads the step counter afresh.
+//  host:           the count uploaded with rcs_set_spawn_counts for this step.
+__device__ __forceinline__ bool ss_wants_spawn(const SourceSinkDev& s, uint32_t k, double dt, const SpawnGenDev& gen) {
+  if (s.gen == GEN_POISSON) return (philox4x64_10_w0(*gen.steps_done + 1ull, k, s.seed) >> 11) >= gen.thr[k];
+  if (s.gen == GEN_HOST) return gen.host_cnt[k] != 0u;
+  return f64_as_usize(round(dt * s.rate)) > 0;  // MonotonicCrowd, source_sink.rs:97-100
+}
+
 // Strips: which of this rank's sources spawn in this step, as a bitmap over the source ids.  The ranks' bitmaps are
 // disjoint (a source is owned by one rank); their sum over the ranks is the global spawn set, from which every rank
 // derives the same sequential ids (lib.rs:128-129: ids follow the order of the source sinks).
-__global__ void ss_flags_kernel(const SourceSinkDev* __restrict__ ss, uint32_t n_ss, double dt,
+__global__ void ss_flags_kernel(const SourceSinkDev* __restrict__ ss, uint32_t n_ss, double dt, SpawnGenDev gen,
                                 const uint32_t* __restrict__ blocked, uint32_t* __restrict__ bits,
                                 const DevStatus* status) {
   if (status->failed) return;
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n_ss) return;
   const SourceSinkDev& s = ss[k];
-  const uint64_t want = f64_as_usize(round(dt * s.rate));  // MonotonicCrowd, source_sink.rs:97-100
-  if (s.alive && s.owned && want > 0 && !blocked[k]) atomicOr(&bits[k >> 5], 1u << (k & 31u));
+  if (s.alive && s.owned && !blocked[k] && ss_wants_spawn(s, k, dt, gen)) atomicOr(&bits[k >> 5], 1u << (k & 31u));
 }
 
 // bits[w] = sum over the ranks' bitmaps (single-process transport; disjoint bits, so the sum is the union)
@@ -1501,12 +1544,17 @@ __global__ void ss_bits_sum_kernel(uint32_t n_words, uint32_t world, const uint3
 // generator asks for >= 1 (the reference's loop over spawn_number is commented out, lib.rs:207-219).
 // Ids are allocated sequentially (lib.rs:128-129) in that order.  gbits != nullptr (strips): the global spawn set
 // (ss_flags_kernel, summed over the ranks) decides and numbers the spawns; this rank materialises its own sources'.
+// Host-generator counts are consumed: cleared on every rank, whether or not the step stands.
 __global__ void ss_spawn_kernel(GridDev g, const SourceSinkDev* __restrict__ ss, const uint32_t* __restrict__ ss_rwp,
-                                uint32_t n_ss, double dt, const uint32_t* __restrict__ gbits,
+                                uint32_t n_ss, double dt, SpawnGenDev gen, const uint32_t* __restrict__ gbits,
                                 uint32_t* __restrict__ blocked, AgentArrays cur, uint32_t* __restrict__ keep,
                                 uint32_t cap, uint32_t* cnt, unsigned long long* next_id, unsigned long long* ev_id, double* ev_xy, uint32_t ev_cap,
                                 DevStatus* status) {
-  if (status->failed) return;
+  if (status->failed) {
+    if (gen.host_cnt)
+      for (uint32_t k = threadIdx.x; k < n_ss; k += blockDim.x) gen.host_cnt[k] = 0u;
+    return;
+  }
   __shared__ uint32_t base_all, base_own;
   if (threadIdx.x == 0) base_all = base_own = 0;
   __syncthreads();
@@ -1521,11 +1569,11 @@ __global__ void ss_spawn_kernel(GridDev g, const SourceSinkDev* __restrict__ ss,
       if (gbits) {
         spawn = (gbits[k >> 5] >> (k & 31u)) & 1u;
       } else {
-        const uint64_t want = f64_as_usize(round(dt * s.rate));  // MonotonicCrowd, source_sink.rs:97-100
-        spawn = (s.alive && want > 0 && !blocked[k]) ? 1u : 0u;
+        spawn = (s.alive && !blocked[k] && ss_wants_spawn(s, k, dt, gen)) ? 1u : 0u;
       }
       mine = (spawn && s.owned) ? 1u : 0u;
       blocked[k] = 0u;
+      if (gen.host_cnt) gen.host_cnt[k] = 0u;
     }
     uint32_t total_all, total_own;
     const uint32_t rank_all = block_exclusive_scan(spawn, total_all);

@@ -175,6 +175,10 @@ class NoHighLevelPlan(HighLevelPlanner):
 
 # ---- source sinks ----------------------------------------------------------------------------
 class CrowdGenerator:
+    """source_sink.rs:63-66.  Subclass and override get_number_to_spawn to run a generator on the host: the simulation
+    calls it once per step for every alive source sink that has it (in ascending source-sink id) and uploads the counts
+    before the step.  Only "at least one" matters: a source spawns at most one agent per step (lib.rs:207-219)."""
+
     def get_number_to_spawn(self, time_elapsed: Duration) -> int:
         raise NotImplementedError
 
@@ -191,6 +195,21 @@ class MonotonicCrowd(CrowdGenerator):
             return 0
         r = np.floor(x)
         return int(r + 1) if x - r >= 0.5 else int(r)
+
+
+class PoissonCrowd(CrowdGenerator):
+    """source_sink.rs:63-82, drawn on the device with a keyed generator instead of thread_rng, so that runs are
+    reproducible.  `seed` is an addition to the reference's constructor.  Source sink `sid` wants to spawn in the step
+    that starts with stats().steps == k iff (word 0 of Philox4x64-10, counter (k + 1, sid, 0, 0), key (seed, 0)) >> 11
+    >= ceil(exp(-dt * rate) * 2^53): probability 1 - exp(-dt * rate) = P(Poisson(dt * rate) >= 1).  rate must be finite
+    and > 0, and a step with dt * rate <= 0 is refused (Poisson::new fails in the reference)."""
+
+    def __init__(self, rate: float, seed: int = 0):
+        self.rate = float(rate)
+        self.seed = int(seed)
+
+    def get_number_to_spawn(self, time_elapsed: Duration) -> int:
+        raise NotImplementedError("PoissonCrowd is drawn on the device inside Simulation.step")
 
 
 @dataclass
@@ -329,6 +348,7 @@ class Simulation:
         self._listeners: Dict[int, EventListener] = {}
         self._listener_counter = 0
         self._source_sinks: Dict[int, SourceSink] = {}
+        self._host_gen: Dict[int, CrowdGenerator] = {}  # source-sink id -> generator evaluated on the host
         self.sim_time = Duration(0, 0)  # never advanced by the reference (lib.rs:81,110)
 
     # -- planner registration ------------------------------------------------------------------
@@ -392,9 +412,17 @@ class Simulation:
     # -- lib.rs:159-173 ------------------------------------------------------------------------
     def add_source_sink(self, source_sink: SourceSink) -> int:
         wp = _f64(source_sink.waypoints).reshape(-1, 2)
-        rate = getattr(source_sink.crowd_generator, "rate", None)
-        if not isinstance(source_sink.crowd_generator, MonotonicCrowd) or rate is None:
-            raise CrowdsimError(N.RCS_ERR_ARG, "only MonotonicCrowd generators run on the device")
+        gen = source_sink.crowd_generator
+        if not isinstance(gen, CrowdGenerator):
+            raise CrowdsimError(N.RCS_ERR_ARG, "the crowd generator must be a CrowdGenerator")
+        if isinstance(gen, MonotonicCrowd):
+            gdesc, rate = None, gen.rate
+        elif isinstance(gen, PoissonCrowd):
+            if not 0 <= gen.seed < 1 << 64:
+                raise CrowdsimError(N.RCS_ERR_ARG, "PoissonCrowd: the seed must lie in [0, 2^64)")
+            gdesc, rate = N.CrowdGeneratorDesc(N.RCS_CROWD_POISSON, 0, gen.rate, gen.seed), 0.0
+        else:  # a user-implemented generator: evaluated on the host before every step (_run_host_generators)
+            gdesc, rate = N.CrowdGeneratorDesc(N.RCS_CROWD_HOST, 0, 0.0, 0), 0.0
         desc = N.SourceSinkDesc(float(source_sink.source[0]), float(source_sink.source[1]),
                                 float(source_sink.radius_sink), float(rate),
                                 self._hl(source_sink.high_level_planner), self._lp(source_sink.local_planner),
@@ -409,14 +437,20 @@ class Simulation:
                 raise CrowdsimError(N.RCS_ERR_ARG, "two source sinks with host-evaluated HighLevelPlanners share a "
                                                    "source position")
         out = C.c_uint64()
-        N.check(self._h, self._lib.rcs_add_source_sink(self._h, C.byref(desc), C.byref(out)))
+        if gdesc is None:
+            N.check(self._h, self._lib.rcs_add_source_sink(self._h, C.byref(desc), C.byref(out)))
+        else:
+            N.check(self._h, self._lib.rcs_add_source_sink_gen(self._h, C.byref(desc), C.byref(gdesc), C.byref(out)))
         self._source_sinks[out.value] = source_sink
+        if gdesc is not None and gdesc.kind == N.RCS_CROWD_HOST:
+            self._host_gen[out.value] = gen
         if host_key is not None:
             self._host_ss[host_key] = source_sink
         return out.value
 
     def remove_source_sink(self, id: int) -> None:
         N.check(self._h, self._lib.rcs_remove_source_sink(self._h, int(id)))
+        self._host_gen.pop(int(id), None)
         ss = self._source_sinks.pop(int(id), None)
         if ss is not None:
             self._host_ss.pop((float(ss.source[0]), float(ss.source[1])), None)
@@ -442,6 +476,7 @@ class Simulation:
     def step(self, dur: Duration) -> None:
         """Err(String) of the reference becomes CrowdsimError with the same message."""
         before = self._run_host_planners() if self._host_hl else None
+        self._run_host_generators(dur)
         N.check(self._h, self._lib.rcs_step(self._h, int(dur.secs), int(dur.nanos)))
         self._dispatch_events(before)
 
@@ -466,10 +501,21 @@ class Simulation:
 
     def step_async(self, dur: Duration, no_commit: bool = False) -> None:
         flags = N.RCS_STEP_NO_COMMIT if no_commit else N.RCS_STEP_DEFAULT
+        self._run_host_generators(dur)
         N.check(self._h, self._lib.rcs_step_async(self._h, int(dur.secs), int(dur.nanos), flags))
 
     def sync(self) -> None:
         N.check(self._h, self._lib.rcs_sync(self._h))
+
+    def _run_host_generators(self, dur: Duration) -> None:
+        """get_number_to_spawn(dur) of every alive host-evaluated CrowdGenerator, in ascending source-sink id, uploaded
+        as the counts of the next step (rcs_set_spawn_counts)."""
+        if not self._host_gen:
+            return
+        ids = sorted(self._host_gen)
+        counts = _u64([int(self._host_gen[i].get_number_to_spawn(dur)) for i in ids])
+        ids = _u64(ids)
+        N.check(self._h, self._lib.rcs_set_spawn_counts(self._h, len(ids), _p(ids, N.c_u64p), _p(counts, N.c_u64p)))
 
     def _run_host_planners(self) -> Dict[str, np.ndarray]:
         """Uploads the host planners' preferred velocities; returns the pre-step state it read."""

@@ -17,10 +17,10 @@ import time
 import numpy as np
 
 
-def build(lp_none: bool, device: int = 0, cols: int = 32, rows: int = 256, strip=None):
+def build(lp_none: bool, device: int = 0, cols: int = 32, rows: int = 256, strip=None, generator=None):
     """strip = (rank, world, nccl_id[, peer_gather]): this rank of a strip-partitioned stream.  Every rank holds all source sinks;
     the rank that owns a source's cell column spawns for it (source columns are 65 c + 17 of 2112: never next to a
-    boundary of 2, 4 or 8 equal strips)."""
+    boundary of 2, 4 or 8 equal strips).  generator: the CrowdGenerator of every source (None: MonotonicCrowd(10/s))."""
     from . import sim as S
 
     margin, cell = 32.0, 2.0
@@ -48,7 +48,8 @@ def build(lp_none: bool, device: int = 0, cols: int = 32, rows: int = 256, strip
             route = [(x0 + 40.03, y0 + 3.0), (x0 + 80.07, y0 - 3.0), (x0 + 125.01, y0)]
             hl = S.RouteFollowPlan(route)
             keep.append(hl)
-            sim.add_source_sink(S.SourceSink((x0, y0), 0.6, S.MonotonicCrowd(10.0), hl, lp, [route[-1]], False, 2.0))
+            gen = S.MonotonicCrowd(10.0) if generator is None else generator
+            sim.add_source_sink(S.SourceSink((x0, y0), 0.6, gen, hl, lp, [route[-1]], False, 2.0))
     sim._keep = keep
     return sim, n_src, dom
 

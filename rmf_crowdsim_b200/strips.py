@@ -189,6 +189,8 @@ class LocalStripGroup:
 
     def step(self, dur: S.Duration, no_commit: bool = False, sync: bool = True) -> None:
         flags = N.RCS_STEP_NO_COMMIT if no_commit else N.RCS_STEP_DEFAULT
+        for sm in self.sims:  # every rank's host generators are called; the rank that owns a source decides
+            sm._run_host_generators(dur)
         rc = self._lib.rcs_dist_step_local(self._handles, self.world, int(dur.secs), int(dur.nanos), flags)
         if rc != N.RCS_OK:
             self._raise(rc)
